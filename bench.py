@@ -619,8 +619,35 @@ def parity_check(wl, spec, sd, lat, image, jobs, mean_latent, n=2):
             'source': 'id maps written by the in-forward label jobs of the timed step (label_wide_kernel / label_native_kernel)'}
 
 
-def measure(wl, args, dev, rank, world, steps, warmup, profile_steps, with_e2e=True, with_parity=True):
-    """One workload on this rank: resident `value`, host-buffer `e2e`, per-kernel roofline, parity of the timed path."""
+DUMP_BYTES = 60 << 20        # 64 MB with room for the .npy headers
+
+
+def dump_outputs(path, image, jobs):
+    """`--dump-outputs`: what one step of the timed path returned -- the image, then per labelled layer the cluster-id
+    map (`ids_<layer>`) and the class masks (`masks_<layer>`) -- as float32 `<name>.npy` files of at most DUMP_BYTES in
+    all.  The budget is shared out smallest array first; an array that does not fit whole is stored as a flat sample at
+    indices drawn with seed 0, so two runs with the same arguments sample the same elements."""
+    import numpy
+    arrays = {'image': image}
+    for j in jobs:
+        arrays[f'ids_{j.activation_idx}'] = j.ids_u8
+        arrays[f'masks_{j.activation_idx}'] = j.masks
+    os.makedirs(path, exist_ok=True)
+    left, n_left = DUMP_BYTES // 4, len(arrays)
+    for name, t in sorted(arrays.items(), key=lambda kv: kv[1].numel()):
+        keep = min(t.numel(), left // n_left)
+        a = t.detach().float().cpu().numpy()
+        if keep < a.size:
+            idx = numpy.sort(numpy.random.default_rng(0).choice(a.size, size=keep, replace=False))
+            a = a.reshape(-1)[idx]
+            print(f'--dump-outputs: {name} {list(t.shape)} stored as a sample of {keep} elements', file=sys.stderr)
+        numpy.save(os.path.join(path, f'{name}.npy'), a)
+        left, n_left = left - keep, n_left - 1
+
+
+def measure(wl, args, dev, rank, world, steps, warmup, profile_steps, with_e2e=True, with_parity=True, dump_dir=None):
+    """One workload on this rank: resident `value`, host-buffer `e2e`, per-kernel roofline, parity of the timed path.
+    `dump_dir`: rank 0 writes the outputs of the last timed step there (dump_outputs)."""
     import copy
 
     import torch.distributed as dist
@@ -727,6 +754,8 @@ def measure(wl, args, dev, rank, world, steps, warmup, profile_steps, with_e2e=T
     clocks = sampler.stop(t_begin, t_end) if rank == 0 else None
     res = {'value': world * steps * B / (ms_total / 1e3), 'ms_per_step': ms_total / steps, 'gpu_launches': launches, 'clocks': clocks,
            'stats_allreduce_sum': int(stats.sum().item()), 'batch': B, 'lanes': n_lanes}
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, *lane_out[(steps - 1) % n_lanes])      # step i ran on lane i % n_lanes
 
     # ---------------------------------------------------------------- parity of the timed path (rank 0)
     if with_parity and rank == 0:
@@ -862,7 +891,12 @@ def main():
                     help='--leg dataset: contour stage on the device (sis_contour_stage) or as host tasks')
     ap.add_argument('--leg', default='', choices=['', 'contours', 'dataset_gan', 'dataset'],
                     help='run one of the extra stage benchmarks (rows after the hot path) instead of the headline metric')
+    ap.add_argument('--dump-outputs', default='', metavar='DIR',
+                    help='write the image, id maps and class masks of the last timed step of --config to DIR/<name>.npy '
+                         '(float32, <= 64 MB in all, larger arrays as a fixed seeded sample; rank 0)')
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == 'reference' or args.leg):
+        ap.error('--dump-outputs writes the outputs of the headline measurement (--impl b200, no --leg)')
     args.warmup = max(args.warmup, 3) if args.impl == 'b200' else args.warmup
     wl = WORKLOADS[args.config]
 
@@ -892,7 +926,7 @@ def main():
             dist.destroy_process_group()
         return
 
-    main_res = measure(wl, args, dev, rank, world, args.steps, args.warmup, args.profile_steps)
+    main_res = measure(wl, args, dev, rank, world, args.steps, args.warmup, args.profile_steps, dump_dir=args.dump_outputs)
 
     extra = []
     extra_ids = args.extra_configs if args.extra_configs is not None else ('3,4' if args.config == 2 and not args.batch else '')
