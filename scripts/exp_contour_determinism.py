@@ -25,4 +25,4 @@ for size, sig in ((128, (3, 3, 1, 1)), (256, (3, 3, 1, 1)), (256, (6, 6, 2.5, 2.
             diffs += not same
             if not same:
                 print('  differs at it', it, 'pixels', int((cur[0] != ref[0]).any(-1).sum()), 'flags', cur[1].tolist(), ref[1].tolist(), cur[2], ref[2])
-    print('size', size, sig, 'halve', os.environ.get('SIS_CT_HALVE', '1'), 'runs differing', diffs, 'info', ref[2])
+    print('size', size, sig, 'runs differing', diffs, 'info', ref[2])

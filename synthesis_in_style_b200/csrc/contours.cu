@@ -85,9 +85,7 @@ __device__ __forceinline__ int uf_find(const int32_t* parent, int i) {
 // find with path halving: every visited node is re-pointed at its grandparent (always an ancestor, so concurrent finds and
 // unions stay correct).  Rows of one big region link into chains as long as the region is tall; without this every
 // later find walks them again (measured on the pipeline's masks: outside test 179 -> 110 us, border marking 31 -> 15 us).
-__constant__ int ct_halve = 1;      // SIS_CT_HALVE=0: plain finds (A/B switch)
 __device__ __forceinline__ int uf_find_halve(int32_t* parent, int i) {
-    if (!ct_halve) return uf_find(parent, i);
     while (true) {
         const int p = ((volatile int32_t*)parent)[i];
         if (p == i) return i;
@@ -709,12 +707,6 @@ extern "C" int sis_contour_stage(const uint8_t* const* d_det_masks, const uint8_
     SIS_REQUIRE(size <= 1024, "contour stage: image size %d not supported (a window row must fit 32 word columns: <= 1024)", size);
     SIS_REQUIRE((int64_t)(n_classes * n_det_keys + n_fine_keys) * batch * size * size < (int64_t)1 << 31,
                 "contour stage: %d planes of %d^2 pixels exceed the 32-bit pixel index; split the batch", (n_classes * n_det_keys + n_fine_keys) * batch, size);
-    static int halve_set = -1;
-    if (halve_set < 0) {
-        const char* e = getenv("SIS_CT_HALVE");
-        halve_set = (e && e[0] == '0') ? 0 : 1;
-        SIS_CHECK_CUDA(cudaMemcpyToSymbol(ct_halve, &halve_set, sizeof(int)));
-    }
     static int fill_smem_set = 0;
     if (fill_smem > fill_smem_set) {
         SIS_CHECK_CUDA(cudaFuncSetAttribute(ct_group_fill_kernel<1024, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, fill_smem));

@@ -531,12 +531,6 @@ static int launch_native(const LabelArgs& a, cudaStream_t stream) {
     return SIS_OK;
 }
 
-static int label_split_enabled() {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("SIS_LABEL_SPLIT"); v = (e && e[0] == '0') ? 0 : 1; }
-    return v;
-}
-
 template <int KMAX, bool RGB, int SPLIT>
 static int launch_wide_split(const LabelArgs& a, const ToRgbArgs& g, cudaStream_t stream) {
     constexpr int QPB = 256 / SPLIT, NACC = KMAX * 4 + (RGB ? 12 : 0);
@@ -552,9 +546,10 @@ static int launch_wide_split(const LabelArgs& a, const ToRgbArgs& g, cudaStream_
 
 template <int KMAX, bool RGB>
 static int launch_wide_impl(const LabelArgs& a, const ToRgbArgs& g, cudaStream_t stream) {
-    // fewer than two blocks per SM: split the channels over four thread groups
+    // fewer than two blocks per SM: split the channels over four thread groups (measured, 64^2 maps at batch 32:
+    // 68 -> 59 us, 99 -> 80 us with the ToRGB fused)
     const int64_t quads = (int64_t)a.H * a.W / 4 * a.batch;
-    if (quads / 256 < 2 * kNumSMs && a.C % 4 == 0 && label_split_enabled()) return launch_wide_split<KMAX, RGB, 4>(a, g, stream);
+    if (quads / 256 < 2 * kNumSMs && a.C % 4 == 0) return launch_wide_split<KMAX, RGB, 4>(a, g, stream);
     return launch_wide_split<KMAX, RGB, 1>(a, g, stream);
 }
 template <int KMAX>
@@ -581,11 +576,8 @@ using namespace sis;
 
 namespace sis {
 
-static int64_t wide_min_quads() {
-    static int64_t v = -1;
-    if (v < 0) { const char* e = getenv("SIS_LABEL_WIDE_MIN_QUADS"); v = e ? atoll(e) : (int64_t)kNumSMs * 160; }   // measured: the wide kernel wins from ~24 k quads (64^2 maps at batch 32: 80 -> 67 us)
-    return v;
-}
+// pixel quads from which the wide kernel is used; measured: it wins from ~24 k quads (64^2 maps at batch 32: 80 -> 67 us)
+constexpr int64_t kWideMinQuads = (int64_t)kNumSMs * 160;
 
 int launch_label(const LabelArgs& a_in, int mode, const ToRgbArgs* fuse_rgb, bool* fused, cudaStream_t stream) {
     LabelArgs a = a_in;
@@ -622,7 +614,7 @@ int launch_label(const LabelArgs& a_in, int mode, const ToRgbArgs* fuse_rgb, boo
     // wide path: enough pixel quads to fill the GPU without slicing channels, integer (or no) mask replication,
     // rows that are a multiple of 4 pixels, k small enough for 4 x k register accumulators
     const int64_t quads = (int64_t)h * w / 4 * batch;
-    const bool wide_ok = vec4 && k <= 24 && (size_t)channels * 24 * 8 <= 160 * 1024 && w % 4 == 0 && quads >= wide_min_quads() && ((int64_t)h * w / 4) % 256 == 0 &&
+    const bool wide_ok = vec4 && k <= 24 && (size_t)channels * 24 * 8 <= 160 * 1024 && w % 4 == 0 && quads >= kWideMinQuads && ((int64_t)h * w / 4) % 256 == 0 &&
                          (!a.masks || (int_ratio && ((((uintptr_t)a.masks) & 15) == 0))) &&
                          (!a.ids_u8 || ((((uintptr_t)a.ids_u8) & 3) == 0)) && (!a.margin || ((((uintptr_t)a.margin) & 15) == 0));
     if (wide_ok) {

@@ -4,12 +4,16 @@
 //
 //   y[b,o,p] = d[b,o] * sum_{t,i} Ws[t,o,i] * xs[b,p+t,i],   xs = s[b,i]*x[b,i,p]  (pre-scaled by the producer)
 //
-// GEMM view: M = pixels (128 per tile = a TBxTHxTW box), N = Cout (BN per tile), K = taps*Cin in 64-wide chunks.
-//   A tile  : one TMA 4-D box {64 ch, TW, TH, TB} of the NHWC bf16 plane at the tap-shifted coordinate; the
-//             conv's zero padding is TMA out-of-bounds fill, so there is no im2col buffer and no halo code.
-//   B tile  : one TMA 3-D box {64 ch, BN, 1 tap} of the [tap][Cout][Cin] weight pack (shared by all samples).
-//   MMA     : tcgen05.mma cta_group::1 kind::f16, M=128, N=BN, K=16, operands straight from 128B-swizzled
-//             shared memory, fp32 accumulator in TMEM (double-buffered: 2 x BN columns).
+// GEMM view: M = pixels (128 per tile), N = Cout (BN per tile), K = taps*Cin in BK-wide chunks (BK = 64, or 32 for
+// layers with 32 input channels).
+//   A tile  : per-tap kernel (modconv_tc_kernel): one TMA im2col load of 128 consecutive pixels of the flattened
+//             (b, y, x) output grid per (tap, K chunk), shifted by the tap offset; the conv's zero padding is the
+//             tensor map's out-of-bounds fill.  Halo kernels: one tiled TMA load of the halo of a spatial output tile
+//             per K chunk, which all taps read through shifted operand descriptors.
+//   B tile  : one TMA 3-D box {BK ch, BN (/2 per CTA of a pair), 1 tap} of the [tap][Cout][Cin] weight pack (shared by
+//             all samples).
+//   MMA     : tcgen05.mma kind::f16, M = 128 (single CTA) or 256 (CTA pair, cta_group::2), N = BN, K = 16, operands
+//             straight from swizzled shared memory, fp32 accumulator in TMEM (double-buffered: 2 x BN columns).
 //   Precision: 3-term bf16 split (hi*hi + hi*lo + lo*hi) into the same accumulator (SURVEY.md §7: single-pass
 //             bf16/tf32 operands cannot meet the label criterion; the 3-term split gives ~1e-4 max abs error).
 //   Epilogue: tcgen05.ld 32x32b -> x demod -> + noise -> + bias -> lrelu*sqrt2 -> fp32 NCHW capture + the next
@@ -17,11 +21,10 @@
 //             phase position (transposed conv; blur + activation follow in blur_act_split_kernel).
 //   The stride-2 transposed conv (model.py:251-259) is 4 output-phase sub-GEMMs with 4/2/2/1 taps (no wasted
 //   FLOPs): out[2y'+py, 2x'+px] = sum_{ky = py (mod 2)...} W[ky,kx] x[y' - ky/2, x' - kx/2].
-// Warp roles (192 threads, persistent, static round-robin tile schedule): warp 0 = TMA producer, warp 1 = MMA
-// issuer + TMEM allocator, warps 2-5 = epilogue (TMEM lane quarter = warp_id % 4).
+// Warp roles (320 threads, persistent, static round-robin tile schedule): warp 0 = TMA producer, warp 1 = MMA
+// issuer + TMEM allocator, warps 2-9 = epilogue (TMEM lane quarter = warp_id % 4, two warps per quarter).
 #include <cuda.h>
 #include <cstring>
-#include <cstdlib>
 #include "common.cuh"
 #include "kernels.h"
 #include "modconv_tc.h"
@@ -140,21 +143,22 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr) {
 }
 
 // ------------------------------------------------------------------------------------------------ kernel
+// One sub-GEMM of a launch: the plain conv (one), the 4 output phases of a transposed conv, or its 4 border strips.
 struct TcSubProblem {
     int ntaps;
     short dy[9], dx[9];         // tap offsets (may carry a sub-problem origin: border strips of the transposed conv)
-    signed char widx[9];
-    signed char phase[9];       // 4-phase halo mode (transposed conv, Cout <= 64): output phase py*2+px of every tap
+    signed char widx[9];        // weight pack tap of every tap
+    signed char phase[9];       // 4-phase halo kernels (transposed conv, Cout <= 64): output phase py*2+px of every tap
     int oh, ow;                 // extent of this sub-problem's output grid
-    int ostride, ooff_y, ooff_x;
-    int tiles_y, tiles_x;       // tiled A mode: spatial tiles of the box
-    int tile_begin;
-    int base_dy, base_dx;       // im2col A mode: smallest tap offset (the traversal box starts there); tap offset = d - base
-    int m_tiles;                // im2col A mode: ceil(B*oh*ow / 128) runs of 128 flattened pixels
+    int ostride, ooff_y, ooff_x;   // output pixel = (y * ostride + ooff_y, x * ostride + ooff_x)
+    int tiles_y, tiles_x;       // halo kernels: spatial output tiles of HALO_TH x HALO_TW
+    int tile_begin;             // first tile of this sub-problem (sub-problems one after another, not interleaved)
+    int base_dy, base_dx;       // per-tap kernel: smallest tap offset (the im2col traversal box starts there)
+    int m_tiles;                // per-tap kernel: ceil(B*oh*ow / 128) im2col runs of 128 flattened pixels
 };
 
 // A-operand tensor maps: one (hi, lo) pair per sub-problem (the im2col maps of the 4 transposed-conv phases have
-// different traversal boxes; tiled mode uses pair 0 for everything) and the weight pack maps.
+// different traversal boxes; the halo kernels use pair 0) and the weight pack maps.
 struct TcMaps {
     CUtensorMap a[4][2];
     CUtensorMap w[2];
@@ -162,22 +166,22 @@ struct TcMaps {
 
 struct TcKernelArgs {
     TcSubProblem sub[4];
-    int nsub, total_tiles;
-    int batch, cin, cout, b_tiles, n_tiles, kchunks;
+    int nsub, total_tiles;      // total_tiles counts tiles (single CTAs) or pair tiles (CTA pairs)
+    int batch, cin, cout, b_tiles, kchunks;
     int mode;                   // 0 plain (fused noise + bias [+ activation]), 1 transposed-conv phase (demod only)
     int act;                    // mode 0: apply lrelu(0.2)*sqrt2 (StyledConv) or not (bare ModulatedConv2d)
-    int im2col;                 // A tiles are 128 consecutive pixels of the flattened (b, y, x) output grid (TMA im2col mode)
     int interleave_units;       // > 0: the 4 transposed-conv phases are interleaved, each padded to this many (pair) tiles
     const float* demod; const float* noise; int64_t noise_bstride; float noise_w; const float* bias;
     float* out_f32; int out_h, out_w;
     const float* s_next; bf16* next_hi; bf16* next_lo;
     unsigned int* error;
-    int stages;                 // pipeline depth actually used (<= the configuration's maximum; 0 = maximum): a shallower
-                                // ring leaves shared memory for a co-resident block of another stream's memory-bound kernel
 };
 
 constexpr int BM = 128, UMMA_K = 16;
-constexpr int TC_THREADS = 320;          // warp 0: TMA, warp 1: MMA, warps 2..9: epilogue (two per TMEM lane quarter)
+constexpr int TC_EPI_WARPS = 8;                        // two per TMEM lane quarter
+constexpr int TC_THREADS = 32 * (2 + TC_EPI_WARPS);   // warp 0: TMA, warp 1: MMA, warps 2..9: epilogue
+// output tile of the halo kernels (16 x 8 pixels = one M = 128 tile; see modconv_tc_halo_kernel)
+constexpr int HALO_TH = 16, HALO_TW = 8, HALO_W = HALO_TW + 2, HALO_H = HALO_TH + 2;
 
 // BK = K elements per pipeline stage = one swizzle row (64 -> 128 B rows, 32 -> 64 B rows; measured: the 64 B rows
 // are slower, the L2 -> SM path is request-bound).  CG = tcgen05 cta_group: with CG = 2 a CTA pair computes a
@@ -198,13 +202,13 @@ struct TileCoord { int sub, b0, y0, x0, n0; int p0; bool dummy; bool skip; };
 
 // Tile t of this CTA.  CG = 1: t is a tile index.  CG = 2: t is a PAIR index and `rank` selects the m-tile of the pair
 // (2*mp + rank); an odd m-tile count leaves rank 1 of the last pair with a dummy tile (it recomputes rank 0's tile and
-// stores nothing).
-template <int BN, int TH, int TW, int TB, int CG>
+// stores nothing).  HALO: m-tiles are HALO_TH x HALO_TW spatial tiles; otherwise im2col runs of 128 flattened pixels.
+template <int BN, bool HALO, int CG>
 __device__ __forceinline__ TileCoord decode_tile(const TcKernelArgs& a, int t, int rank) {
     TileCoord c;
     c.skip = false;
     int p = 0, local;
-    if (a.interleave_units) {
+    if (!HALO && a.interleave_units) {
         // transposed conv, im2col mode: the 4 phase sub-GEMMs walk the image together (phase fastest, rotated so a
         // CTA's static stride does not lock onto one phase), so the input planes are read from DRAM once, not 4 times.
         // All phases are padded to the same number of units; the surplus tiles are skipped by every role alike.
@@ -219,24 +223,24 @@ __device__ __forceinline__ TileCoord decode_tile(const TcKernelArgs& a, int t, i
         local = t - a.sub[p].tile_begin;
     }
     const TcSubProblem& s = a.sub[p];
-    const int m_tiles = a.im2col ? s.m_tiles : a.b_tiles * s.tiles_y * s.tiles_x;
-    const int m_units = a.interleave_units ? a.interleave_units : (m_tiles + CG - 1) / CG;
+    const int m_tiles = HALO ? a.b_tiles * s.tiles_y * s.tiles_x : s.m_tiles;
+    const int m_units = (!HALO && a.interleave_units) ? a.interleave_units : (m_tiles + CG - 1) / CG;
     int m = (local % m_units) * CG + rank;
     const int n = local / m_units;
-    if (a.interleave_units && (local % m_units) * CG >= m_tiles) c.skip = true;
+    if (!HALO && a.interleave_units && (local % m_units) * CG >= m_tiles) c.skip = true;
     c.dummy = m >= m_tiles;
     if (c.dummy) m = m_tiles - 1;
     c.sub = p;
-    if (a.im2col) {
+    if (HALO) {
+        c.p0 = 0;
+        c.x0 = (m % s.tiles_x) * HALO_TW;
+        c.y0 = ((m / s.tiles_x) % s.tiles_y) * HALO_TH;
+        c.b0 = m / (s.tiles_x * s.tiles_y);
+    } else {
         c.p0 = m * BM;                              // first flattened pixel of the run
         c.x0 = c.p0 % s.ow;
         c.y0 = (c.p0 / s.ow) % s.oh;
         c.b0 = c.p0 / (s.ow * s.oh);
-    } else {
-        c.p0 = 0;
-        c.x0 = (m % s.tiles_x) * TW;
-        c.y0 = ((m / s.tiles_x) % s.tiles_y) * TH;
-        c.b0 = (m / (s.tiles_x * s.tiles_y)) * TB;
     }
     c.n0 = n * BN;
     return c;
@@ -349,26 +353,26 @@ __device__ __forceinline__ void load32(const float* p, float (&o)[32]) {
 
 // UP4: the accumulator holds the FOUR output phases of a transposed conv side by side (4 x BN columns; phase p of pixel
 // (yy, xx) goes to scratch position (2yy + py, 2xx + px); the py = 1 / px = 1 phases are one row / column shorter).
-template <int BN, int TH, int TW, int TB, int CG, bool UP4 = false>
+template <int BN, bool HALO, int CG, bool UP4 = false>
 __device__ __forceinline__ void tc_epilogue(const TcKernelArgs& a, uint64_t* tfull_bar, uint64_t* tempty_bar, uint32_t tmem_base,
                                             int rank, int warp, int lane, int unit0, int unit_stride) {
         // ============================== epilogue (warps 2..9) ==============================
         const int quarter = warp & 3;                   // TMEM lane quarter this warp may access
         const int chalf = (warp - 2) >> 2;              // the two warps of a quarter take alternate 32-column chunks
-        const int row = quarter * 32 + lane;            // GEMM row = pixel of the tile box
-        const int tw = row % TW, th = (row / TW) % TH, tb = row / (TW * TH);
+        const int row = quarter * 32 + lane;            // GEMM row = pixel of the tile
+        const int tw = row % HALO_TW, th = row / HALO_TW;
         const uint32_t tempty_leader = (CG == 2) ? map_to_cta(smem_u32(&tempty_bar[0]), 0) : 0u;
         int acc = 0; uint32_t acc_phase = 0;
         for (int t = unit0; t < a.total_tiles; t += unit_stride) {
-            const TileCoord c = decode_tile<BN, TH, TW, TB, CG>(a, t, rank);
+            const TileCoord c = decode_tile<BN, HALO, CG>(a, t, rank);
             if (c.skip) continue;
             const TcSubProblem& s = a.sub[c.sub];
             int b, yy, xx;
-            if (a.im2col) {
+            if (HALO) {
+                b = c.b0; yy = c.y0 + th; xx = c.x0 + tw;
+            } else {
                 const int p = c.p0 + row;
                 xx = p % s.ow; yy = (p / s.ow) % s.oh; b = p / (s.ow * s.oh);
-            } else {
-                b = c.b0 + tb; yy = c.y0 + th; xx = c.x0 + tw;
             }
             const bool valid0 = !c.dummy && b < a.batch && yy < s.oh && xx < s.ow;
             const int oy0 = yy * s.ostride + s.ooff_y, ox0 = xx * s.ostride + s.ooff_x;
@@ -379,9 +383,9 @@ __device__ __forceinline__ void tc_epilogue(const TcKernelArgs& a, uint64_t* tfu
             const float* dm = a.demod + (int64_t)(valid0 ? b : 0) * a.cout + c.n0;
             float nz = 0.0f;
             if (!UP4 && a.mode == 0 && valid0 && a.noise) nz = __fmul_rn(a.noise_w, a.noise[(int64_t)b * a.noise_bstride + (int64_t)oy0 * a.out_w + ox0]);
-            const int cstep = (blockDim.x / 32 - 2) * 8;      // 4 epilogue warps: 32, 8: 64
 #pragma unroll 1
-            for (int call = chalf * 32; call < ACC_COLS; call += cstep) {
+            for (int k = chalf; k < ACC_COLS / 32; k += 2) {       // this warp's 32-column chunks
+                const int call = k * 32;
                 const int ph = UP4 ? call / BN : 0;
                 const int c0 = UP4 ? call - ph * BN : call;
                 const bool valid = UP4 ? (valid0 && yy < s.oh - (ph >> 1) && xx < s.ow - (ph & 1)) : valid0;
@@ -449,13 +453,13 @@ __device__ __forceinline__ void tc_epilogue(const TcKernelArgs& a, uint64_t* tfu
         }
     }
 
-template <int BN, int TH, int TW, int TB, int BK, int CG>
+// Per-tap kernel: one im2col A tile per (tap, K chunk).
+template <int BN, int BK, int CG>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 modconv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcKernelArgs a) {
-    static_assert(TH * TW * TB == BM, "tile box must hold 128 pixels");
     static_assert(CG == 1 || CG == 2, "cta_group");
     using Cfg = TcCfg<BN, BK, CG>;
-    const int STAGES = a.stages > 0 && a.stages < Cfg::STAGES ? a.stages : Cfg::STAGES;
+    constexpr int STAGES = Cfg::STAGES;
     constexpr int A_TILE_BYTES = Cfg::A_TILE_BYTES;
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
@@ -476,7 +480,7 @@ modconv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ T
         for (int i = 0; i < a.nsub; ++i) { tma_prefetch_desc(&maps.a[i][0]); tma_prefetch_desc(&maps.a[i][1]); }
         tma_prefetch_desc(&maps.w[0]); tma_prefetch_desc(&maps.w[1]);
         for (int i = 0; i < STAGES; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1); }
-        for (int i = 0; i < 2; ++i) { mbar_init(&tfull_bar[i], 1); mbar_init(&tempty_bar[i], (blockDim.x / 32 - 2) * CG); }
+        for (int i = 0; i < 2; ++i) { mbar_init(&tfull_bar[i], 1); mbar_init(&tempty_bar[i], TC_EPI_WARPS * CG); }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 1) {
@@ -498,14 +502,14 @@ modconv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ T
         {
             int stage = 0; uint32_t phase = 0;
             for (int t = unit0; t < a.total_tiles; t += unit_stride) {
-                const TileCoord c = decode_tile<BN, TH, TW, TB, CG>(a, t, rank);
+                const TileCoord c = decode_tile<BN, false, CG>(a, t, rank);
                 if (c.skip) continue;
                 const TcSubProblem& s = a.sub[c.sub];
                 const int wrow = c.n0 + rank * Cfg::B_ROWS;
-                const CUtensorMap* ma_hi = &maps.a[a.im2col ? c.sub : 0][0];
-                const CUtensorMap* ma_lo = &maps.a[a.im2col ? c.sub : 0][1];
+                const CUtensorMap* ma_hi = &maps.a[c.sub][0];
+                const CUtensorMap* ma_lo = &maps.a[c.sub][1];
                 for (int tap = 0; tap < s.ntaps; ++tap) {
-                    const int ax = c.x0 + s.dx[tap], ay = c.y0 + s.dy[tap], wi = s.widx[tap];
+                    const int wi = s.widx[tap];
                     const unsigned short ow_ = (unsigned short)(s.dx[tap] - s.base_dx), oh_ = (unsigned short)(s.dy[tap] - s.base_dy);
                     for (int kc = 0; kc < a.kchunks; ++kc) {
                         mbar_wait(&empty_bar[stage], phase ^ 1, a.error, 0x100 + stage);
@@ -513,13 +517,8 @@ modconv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ T
                         if (elect_one()) {
                             // one arming per stage: the even CTA expects the bytes of BOTH CTAs on its barrier
                             if (leader) mbar_expect_tx(&full_bar[stage], CG * Cfg::STAGE_BYTES);
-                            if (a.im2col) {
-                                tma_load_im2col_cg<CG>(ma_hi, &full_bar[stage], st, kc * BK, c.x0 + s.base_dx, c.y0 + s.base_dy, c.b0, ow_, oh_);
-                                tma_load_im2col_cg<CG>(ma_lo, &full_bar[stage], st + A_TILE_BYTES, kc * BK, c.x0 + s.base_dx, c.y0 + s.base_dy, c.b0, ow_, oh_);
-                            } else {
-                                tma_load_4d_cg<CG>(ma_hi, &full_bar[stage], st, kc * BK, ax, ay, c.b0);
-                                tma_load_4d_cg<CG>(ma_lo, &full_bar[stage], st + A_TILE_BYTES, kc * BK, ax, ay, c.b0);
-                            }
+                            tma_load_im2col_cg<CG>(ma_hi, &full_bar[stage], st, kc * BK, c.x0 + s.base_dx, c.y0 + s.base_dy, c.b0, ow_, oh_);
+                            tma_load_im2col_cg<CG>(ma_lo, &full_bar[stage], st + A_TILE_BYTES, kc * BK, c.x0 + s.base_dx, c.y0 + s.base_dy, c.b0, ow_, oh_);
                             tma_load_3d_cg<CG>(&maps.w[0], &full_bar[stage], st + 2 * A_TILE_BYTES, kc * BK, wrow, wi);
                             tma_load_3d_cg<CG>(&maps.w[1], &full_bar[stage], st + 2 * A_TILE_BYTES + Cfg::B_TILE_BYTES, kc * BK, wrow, wi);
                         }
@@ -537,7 +536,7 @@ modconv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ T
             int stage = 0; uint32_t phase = 0;
             int acc = 0; uint32_t acc_phase = 0;
             for (int t = unit0; t < a.total_tiles; t += unit_stride) {
-                const TileCoord c = decode_tile<BN, TH, TW, TB, CG>(a, t, 0);
+                const TileCoord c = decode_tile<BN, false, CG>(a, t, 0);
                 if (c.skip) continue;
                 const int kblocks = a.sub[c.sub].ntaps * a.kchunks;
                 mbar_wait(&tempty_bar[acc], acc_phase ^ 1, a.error, 0x200 + acc);
@@ -568,7 +567,7 @@ modconv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ T
             }
         }
     } else {
-        tc_epilogue<BN, TH, TW, TB, CG>(a, tfull_bar, tempty_bar, tmem_base, rank, warp, lane, unit0, unit_stride);
+        tc_epilogue<BN, false, CG>(a, tfull_bar, tempty_bar, tmem_base, rank, warp, lane, unit0, unit_stride);
     }
     tc_fence_before();
     if (CG == 2) cluster_sync_all(); else __syncthreads();   // CG = 2: the peer may still read this CTA's smem / TMEM
@@ -590,7 +589,6 @@ modconv_tc_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ T
 // inside a 1024 B-aligned TMA-written buffer reads back consistently with base_offset 0 (scripts/exp_halo_desc.cu
 // verifies this on the B200).  A traffic drops from 9 x 32 KB to 45 KB per K chunk; the weights stream per tap through
 // their own ring.  With Cout = 128 that takes the L2 -> SM fill from ~62 to ~27 B/clk/SM, i.e. back under the tensor pipe.
-constexpr int HALO_TH = 16, HALO_TW = 8, HALO_W = HALO_TW + 2, HALO_H = HALO_TH + 2;
 // BK = 64: 128 B operand rows (SWIZZLE_128B); BK = 32 (layers with 32 input channels): 64 B rows (SWIZZLE_64B), as the
 // transposed halo kernel below uses them.
 // UP4 (transposed conv with Cout <= 64): the 9 taps of a stride-2 transposed conv fall into 4 output phases with 4/2/2/1
@@ -633,7 +631,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1)
 modconv_tc_halo_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcKernelArgs a) {
     using Cfg = TcHaloCfg<BN, CG, BK, UP4>;
     constexpr int NA = Cfg::NA, ROW = Cfg::ROW;
-    const int NB = a.stages > 0 && a.stages < Cfg::NB ? a.stages : Cfg::NB;
+    constexpr int NB = Cfg::NB;
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
     uint8_t* smem_b = smem + NA * Cfg::A_STAGE;
@@ -657,7 +655,7 @@ modconv_tc_halo_kernel(const __grid_constant__ TcMaps maps, const __grid_constan
         tma_prefetch_desc(&maps.w[0]); tma_prefetch_desc(&maps.w[1]);
         for (int i = 0; i < NB; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1); }
         for (int i = 0; i < NA; ++i) { mbar_init(&afull_bar[i], 1); mbar_init(&aempty_bar[i], 1); }
-        for (int i = 0; i < 2; ++i) { mbar_init(&tfull_bar[i], 1); mbar_init(&tempty_bar[i], (blockDim.x / 32 - 2) * CG); }
+        for (int i = 0; i < 2; ++i) { mbar_init(&tfull_bar[i], 1); mbar_init(&tempty_bar[i], TC_EPI_WARPS * CG); }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 1) {
@@ -681,7 +679,7 @@ modconv_tc_halo_kernel(const __grid_constant__ TcMaps maps, const __grid_constan
             int as = 0; uint32_t aphase = 0;
             int bs = 0; uint32_t bphase = 0;
             for (int t = unit0; t < a.total_tiles; t += unit_stride) {
-                const TileCoord c = decode_tile<BN, HALO_TH, HALO_TW, 1, CG>(a, t, rank);
+                const TileCoord c = decode_tile<BN, true, CG>(a, t, rank);
                 const int wrow = c.n0 + rank * Cfg::B_ROWS;
                 for (int kc = 0; kc < a.kchunks; ++kc) {
                     mbar_wait(&aempty_bar[as], aphase ^ 1, a.error, 0x500 + as);
@@ -756,7 +754,7 @@ modconv_tc_halo_kernel(const __grid_constant__ TcMaps maps, const __grid_constan
             }
         }
     } else {
-        tc_epilogue<BN, HALO_TH, HALO_TW, 1, CG, UP4>(a, tfull_bar, tempty_bar, tmem_base, rank, warp, lane, unit0, unit_stride);
+        tc_epilogue<BN, true, CG, UP4>(a, tfull_bar, tempty_bar, tmem_base, rank, warp, lane, unit0, unit_stride);
     }
     tc_fence_before();
     if (CG == 2) cluster_sync_all(); else __syncthreads();
@@ -817,7 +815,7 @@ modconv_tc_halo_rw_kernel(const __grid_constant__ TcMaps maps, const __grid_cons
         tma_prefetch_desc(&maps.a[0][0]); tma_prefetch_desc(&maps.a[0][1]);
         tma_prefetch_desc(&maps.w[0]); tma_prefetch_desc(&maps.w[1]);
         for (int i = 0; i < NA; ++i) { mbar_init(&afull_bar[i], 1); mbar_init(&aempty_bar[i], 1); }
-        for (int i = 0; i < 2; ++i) { mbar_init(&tfull_bar[i], 1); mbar_init(&tempty_bar[i], blockDim.x / 32 - 2); }
+        for (int i = 0; i < 2; ++i) { mbar_init(&tfull_bar[i], 1); mbar_init(&tempty_bar[i], TC_EPI_WARPS); }
         mbar_init(wfull_bar, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
@@ -843,7 +841,7 @@ modconv_tc_halo_rw_kernel(const __grid_constant__ TcMaps maps, const __grid_cons
         __syncwarp();
         int as = 0; uint32_t aphase = 0;
         for (int t = unit0; t < a.total_tiles; t += unit_stride) {
-            const TileCoord c = decode_tile<BN, HALO_TH, HALO_TW, 1, 1>(a, t, 0);
+            const TileCoord c = decode_tile<BN, true, 1>(a, t, 0);
             mbar_wait(&aempty_bar[as], aphase ^ 1, a.error, 0x500 + as);
             uint8_t* sa = smem_a + as * Cfg::A_STAGE;
             if (elect_one()) {
@@ -895,7 +893,7 @@ modconv_tc_halo_rw_kernel(const __grid_constant__ TcMaps maps, const __grid_cons
             if (++acc == 2) { acc = 0; acc_phase ^= 1; }
         }
     } else {
-        tc_epilogue<BN, HALO_TH, HALO_TW, 1, 1, UP4>(a, tfull_bar, tempty_bar, tmem_base, 0, warp, lane, unit0, unit_stride);
+        tc_epilogue<BN, true, 1, UP4>(a, tfull_bar, tempty_bar, tmem_base, 0, warp, lane, unit0, unit_stride);
     }
     tc_fence_before();
     __syncthreads();
@@ -958,7 +956,6 @@ modconv_tc_halo_t_kernel(const __grid_constant__ TcMaps maps, const __grid_const
     uint32_t* tmem_ptr_smem = (uint32_t*)(tempty_bar + 2);
 
     const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;   // provably warp-uniform
-    const int n_epi_warps = (int)(blockDim.x / 32) - 2;
     // tiles: n-tile slowest, then spatial tile, then (transposed conv) the 4 output phases, rotated by the spatial index so
     // that a CTA's static stride (148 = 4 * 37) does not lock onto one phase (they have 4 / 2 / 2 / 1 taps)
     const int tiles_x = a.sub[0].ow / HT_TW, tiles_y = a.sub[0].oh / HT_TH;
@@ -970,7 +967,7 @@ modconv_tc_halo_t_kernel(const __grid_constant__ TcMaps maps, const __grid_const
         tma_prefetch_desc(&maps.w[0]); tma_prefetch_desc(&maps.w[1]);
         for (int i = 0; i < NW; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1); }
         for (int i = 0; i < NA; ++i) { mbar_init(&afull_bar[i], 1); mbar_init(&aempty_bar[i], 1); }
-        for (int i = 0; i < 2; ++i) { mbar_init(&tfull_bar[i], 1); mbar_init(&tempty_bar[i], n_epi_warps); }
+        for (int i = 0; i < 2; ++i) { mbar_init(&tfull_bar[i], 1); mbar_init(&tempty_bar[i], TC_EPI_WARPS); }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 1) {
@@ -1066,7 +1063,6 @@ modconv_tc_halo_t_kernel(const __grid_constant__ TcMaps maps, const __grid_const
         // ============================== epilogue: one output channel per thread ==============================
         const int quarter = warp & 3;
         const int chalf = (warp - 2) >> 2;
-        const int cstep = n_epi_warps * 8;                  // 4 epilogue warps: 32 columns, 8: 64
         int acc = 0; uint32_t acc_phase = 0;
         for (int t = blockIdx.x; t < a.total_tiles; t += gridDim.x) {
             const int rt = t % (m_tiles * per), n0 = (t / (m_tiles * per)) * 128;
@@ -1083,7 +1079,7 @@ modconv_tc_halo_t_kernel(const __grid_constant__ TcMaps maps, const __grid_const
             tc_fence_after();
             const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(acc * HT_N);
 #pragma unroll 1
-            for (int c0 = chalf * 32; c0 < HT_N; c0 += cstep) {
+            for (int c0 = chalf * 32; c0 < HT_N; c0 += 64) {
                 uint32_t r[32];
                 tmem_ld_32x32(taddr + (uint32_t)c0, r);
                 tmem_ld_wait();
@@ -1180,11 +1176,6 @@ template <int CB> struct BlurGeo {
     static_assert(CB * OPITCH * 4 <= SMEM, "the transposed output must fit in the input tile");
 };
 
-__device__ __forceinline__ void cp_async_16(void* smem_dst, const void* gmem_src) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(smem_dst)), "l"(gmem_src) : "memory");
-}
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
-
 // packed fp32x2 arithmetic (sm_100: FFMA2 / FADD2 / FMUL2): two channels per lane per instruction
 using u64 = unsigned long long;
 __device__ __forceinline__ float2 ffma2(float2 a, float2 b, float2 c) {
@@ -1225,20 +1216,18 @@ __device__ __forceinline__ void sts_f1(uint32_t addr, float v) { asm volatile("s
 // `blur.kernel` takes the generic 16-tap path.  The bf16 hi/lo NHWC planes are written straight from registers; the fp32
 // NCHW capture goes through a shared-memory transpose that re-uses the input tile's storage.  All index arithmetic is
 // hoisted out of the per-element loops: the kernel is HBM-bound only if its instruction count is small.
-// RING > 0: the input tile comes from ONE TMA box load (fp32 NHWC scratch, out-of-bounds rows / columns / channels are
-// zero-filled by the tensor map) into a ring, issued a tile ahead by thread 0: no per-thread staging instructions and the
-// load of tile i+1 overlaps the math and stores of tile i.  RING = 0 (cp.async staging) exists for CB = 64 only.
-template <bool SEP, int RING, int CB>     // RING: 0 = cp.async staging, 1 / 2 = TMA ring depth
-__global__ void __launch_bounds__(256, RING == 2 ? 2 : 3) blur_act_split_kernel(BlurSplitArgs a, const __grid_constant__ CUtensorMap in_map) {
+// The input tile comes from ONE TMA box load (fp32 NHWC scratch, out-of-bounds rows / columns / channels are zero-filled
+// by the tensor map) into a ring of two, issued a tile ahead by thread 0: no per-thread staging instructions and the load
+// of tile i+1 overlaps the math and stores of tile i.
+template <bool SEP, int CB>
+__global__ void __launch_bounds__(256, 2) blur_act_split_kernel(BlurSplitArgs a, const __grid_constant__ CUtensorMap in_map) {
     using G = BlurGeo<CB>;
-    constexpr bool TMA = RING > 0;
     constexpr int TW = G::TW, IW = G::IW, LPG = G::LPG, OPITCH = G::OPITCH, TILE_BYTES = G::SMEM;
-    static_assert(TMA || CB == 64, "cp.async staging is only written for 64-channel blocks");
-    extern __shared__ __align__(128) float stile_raw[];    // [11*IW][CB] fp32 (x2 with TMA); re-used as sout[CB][OPITCH]
+    extern __shared__ __align__(128) float stile_raw[];    // 2 x [11*IW][CB] fp32; a slot is re-used as sout[CB][OPITCH]
     __shared__ float sk[16], skx[4], sky[4];
     __shared__ float snz[BS_TH * TW];
     __shared__ uint64_t tma_bar[2];
-    float* stile = TMA ? (float*)(((uintptr_t)stile_raw + 127) & ~(uintptr_t)127) : stile_raw;
+    float* const ring0 = (float*)(((uintptr_t)stile_raw + 127) & ~(uintptr_t)127);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int grp = lane / LPG, cl = lane - grp * LPG;      // column-pair group of this lane, channel pair inside the block
     if (tid < 16) sk[tid] = a.blur_k[(3 - tid / 4) * 4 + (3 - tid % 4)];   // flipped taps
@@ -1247,8 +1236,6 @@ __global__ void __launch_bounds__(256, RING == 2 ? 2 : 3) blur_act_split_kernel(
     const int tiles_x = (a.OW + TW - 1) / TW, tiles_y = (a.OH + BS_TH - 1) / BS_TH;
     const int cgroups = (a.C + CB - 1) / CB;
     const int64_t total = (int64_t)a.batch * tiles_y * tiles_x * cgroups;
-    const int part = tid & 15;
-    float* const ring0 = stile;
     auto tile_coords = [&](int64_t tile, int& b, int& y0, int& x0, int& c0) {
         const int cg = (int)(tile % cgroups);
         int64_t r = tile / cgroups;
@@ -1256,66 +1243,36 @@ __global__ void __launch_bounds__(256, RING == 2 ? 2 : 3) blur_act_split_kernel(
         const int ty = (int)(r % tiles_y);
         b = (int)(r / tiles_y); y0 = ty * BS_TH; x0 = tx * TW; c0 = cg * CB;
     };
-    if (TMA) {
-        if (tid == 0) {
-            mbar_init(&tma_bar[0], 1); mbar_init(&tma_bar[1], 1);
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-            if (RING == 2 && (int64_t)blockIdx.x < total) {
-                int b, y0, x0, c0;
-                tile_coords(blockIdx.x, b, y0, x0, c0);
-                mbar_expect_tx(&tma_bar[0], TILE_BYTES);
-                tma_load_4d(&in_map, &tma_bar[0], ring0, c0, x0 - 1, y0 - 1, b);
-            }
+    if (tid == 0) {
+        mbar_init(&tma_bar[0], 1); mbar_init(&tma_bar[1], 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        if ((int64_t)blockIdx.x < total) {
+            int b, y0, x0, c0;
+            tile_coords(blockIdx.x, b, y0, x0, c0);
+            mbar_expect_tx(&tma_bar[0], TILE_BYTES);
+            tma_load_4d(&in_map, &tma_bar[0], ring0, c0, x0 - 1, y0 - 1, b);
         }
     }
     int it = 0;
     for (int64_t tile = blockIdx.x; tile < total; tile += gridDim.x, ++it) {
         int b, y0, x0, c0;
         tile_coords(tile, b, y0, x0, c0);
-        if (RING == 2) stile = ring0 + (it & 1) * (TILE_BYTES / 4);
+        float* const stile = ring0 + (it & 1) * (TILE_BYTES / 4);
         const uint32_t stile_u32 = smem_u32(stile);                    // tile: [pix][CB / 2 lanes] float2
         __syncthreads();     // previous tile's transpose reads are done (and the tap tables are visible)
-        if (TMA) {
-            // the other ring slot held the previous tile (its transposed output was just consumed): refill it a tile ahead
-            if (RING == 2 && tid == 0 && tile + gridDim.x < total) {
-                int nb, ny0, nx0, nc0;
-                tile_coords(tile + gridDim.x, nb, ny0, nx0, nc0);
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");     // generic-proxy accesses of that slot are done
-                mbar_expect_tx(&tma_bar[(it + 1) & 1], TILE_BYTES);
-                tma_load_4d(&in_map, &tma_bar[(it + 1) & 1], ring0 + ((it + 1) & 1) * (TILE_BYTES / 4), nc0, nx0 - 1, ny0 - 1, nb);
-            }
-            if (RING == 1 && tid == 0) {
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                mbar_expect_tx(&tma_bar[0], TILE_BYTES);
-                tma_load_4d(&in_map, &tma_bar[0], ring0, c0, x0 - 1, y0 - 1, b);
-            }
-            if (tid < BS_TH * TW) {
-                const int oy = y0 + tid / TW, ox = x0 + tid % TW;
-                snz[tid] = (a.noise && oy < a.OH && ox < a.OW) ? a.noise_w * __ldg(a.noise + (int64_t)b * a.noise_bstride + (int64_t)oy * a.OW + ox) : 0.0f;
-            }
-            if (RING == 2) mbar_wait(&tma_bar[it & 1], (uint32_t)((it >> 1) & 1), nullptr, 0);
-            else mbar_wait(&tma_bar[0], (uint32_t)(it & 1), nullptr, 0);
-        } else {
-        // ---- stage the input tile: 16 threads per pixel (16-byte parts), 16 pixels per pass
-        {
-            const float* src_base = a.in + (int64_t)b * a.IH * a.IW * a.C + c0 + part * 4;
-#pragma unroll 2
-            for (int pi = tid >> 4; pi < BS_IH * IW; pi += 16) {
-                const int ry = pi / IW, rx = pi - ry * IW;
-                const int iy = y0 + ry - 1, ix = x0 + rx - 1;
-                const uint32_t dst = stile_u32 + (uint32_t)(pi * CB + part * 4) * 4u;
-                if ((unsigned)iy < (unsigned)a.IH && (unsigned)ix < (unsigned)a.IW && c0 + part * 4 < a.C)
-                    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src_base + (int64_t)(iy * a.IW + ix) * a.C) : "memory");
-                else
-                    asm volatile("st.shared.v4.f32 [%0], {%1, %1, %1, %1};" ::"r"(dst), "f"(0.0f) : "memory");
-            }
-            if (tid < BS_TH * TW) {
-                const int oy = y0 + tid / TW, ox = x0 + tid % TW;
-                snz[tid] = (a.noise && oy < a.OH && ox < a.OW) ? a.noise_w * __ldg(a.noise + (int64_t)b * a.noise_bstride + (int64_t)oy * a.OW + ox) : 0.0f;
-            }
+        // the other ring slot held the previous tile (its transposed output was just consumed): refill it a tile ahead
+        if (tid == 0 && tile + gridDim.x < total) {
+            int nb, ny0, nx0, nc0;
+            tile_coords(tile + gridDim.x, nb, ny0, nx0, nc0);
+            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");     // generic-proxy accesses of that slot are done
+            mbar_expect_tx(&tma_bar[(it + 1) & 1], TILE_BYTES);
+            tma_load_4d(&in_map, &tma_bar[(it + 1) & 1], ring0 + ((it + 1) & 1) * (TILE_BYTES / 4), nc0, nx0 - 1, ny0 - 1, nb);
         }
-        cp_async_wait_all();
+        if (tid < BS_TH * TW) {
+            const int oy = y0 + tid / TW, ox = x0 + tid % TW;
+            snz[tid] = (a.noise && oy < a.OH && ox < a.OW) ? a.noise_w * __ldg(a.noise + (int64_t)b * a.noise_bstride + (int64_t)oy * a.OW + ox) : 0.0f;
         }
+        mbar_wait(&tma_bar[it & 1], (uint32_t)((it >> 1) & 1), nullptr, 0);
         __syncthreads();
 
         // ---- blur: column pair (px, px+1), rows top to bottom
@@ -1594,19 +1551,6 @@ static int make_im2col_map(CUtensorMap* map, void* base, int C, int W, int H, in
     return SIS_OK;
 }
 
-struct TcTensorMapCacheEntry { CUtensorMap m; };
-
-static int env_int(const char* name, int dflt) {
-    const char* e = getenv(name);
-    return e ? atoi(e) : dflt;
-}
-// SIS_TC_EPIWARPS (8 default | 4): epilogue warps per CTA; the kernels size their barriers from blockDim
-static int tc_threads() {
-    static int t = 0;
-    if (!t) t = env_int("SIS_TC_EPIWARPS", 8) == 4 ? 192 : TC_THREADS;
-    return t;
-}
-
 int tc_pack_weights(TcConvWeights& w, const float* d_weight, int cin, int cout, bool up, float scale, cudaStream_t stream) {
     (void)up;
     const size_t bytes = (size_t)9 * cin * cout * sizeof(bf16);
@@ -1659,8 +1603,6 @@ void tc_free_workspace(TcWorkspace& ws) {
         ws.a_hi[i] = ws.a_lo[i] = nullptr;
     }
     ws.d_error = nullptr; ws.a_bytes = 0; ws.batch = -1;      // the watchdog word belongs to the library
-    for (auto* e : ws.maps) delete e;
-    ws.maps.clear();
 }
 
 int tc_check_error(TcWorkspace& ws, cudaStream_t stream) {
@@ -1682,147 +1624,170 @@ int tc_prescale_split(TcWorkspace& ws, int slot, const float* x, const float* s,
     return SIS_OK;
 }
 
-template <int BN, int TH, int TW, int TB, int BK, int CG>
-static int launch_tc(const TcMaps& maps, const TcKernelArgs& a, cudaStream_t stream) {
-    using Cfg = TcCfg<BN, BK, CG>;
-    auto kern = modconv_tc_kernel<BN, TH, TW, TB, BK, CG>;
+// Weight pack maps: boxes of {BK channels, `rows` output channels, 1 tap} of the [taps][Cout][Cin] hi / lo packs.
+static int make_weight_maps(TcMaps& maps, const void* hi, const void* lo, int cin, int cout, int taps, int BK, int rows) {
+    const uint64_t wdims[3] = {(uint64_t)cin, (uint64_t)cout, (uint64_t)taps};
+    const uint32_t wbox[3] = {(uint32_t)BK, (uint32_t)rows, 1};
+    SIS_PROPAGATE(make_map(&maps.w[0], const_cast<void*>(hi), 3, wdims, wbox, BK * 2));
+    SIS_PROPAGATE(make_map(&maps.w[1], const_cast<void*>(lo), 3, wdims, wbox, BK * 2));
+    return SIS_OK;
+}
+
+// Halo maps of the conv's input planes: boxes of {BK channels, hw x hh pixels, 1 sample}; the out-of-bounds zero fill is
+// the conv's padding.
+static int make_halo_maps(TcMaps& maps, const TcWorkspace& ws, const TcConvCall& call, int BK, int hw, int hh) {
+    const uint64_t adims[4] = {(uint64_t)call.cin, (uint64_t)call.res_in, (uint64_t)call.res_in, (uint64_t)call.batch};
+    const uint32_t abox[4] = {(uint32_t)BK, (uint32_t)hw, (uint32_t)hh, 1};
+    SIS_PROPAGATE(make_map(&maps.a[0][0], ws.a_hi[call.in_slot], 4, adims, abox, BK * 2));
+    SIS_PROPAGATE(make_map(&maps.a[0][1], ws.a_lo[call.in_slot], 4, adims, abox, BK * 2));
+    return SIS_OK;
+}
+
+// im2col maps of sub-problem i over the conv's input planes: the base pixels of its runs span the traversal box
+// [base_d, base_d + extent - 1] = [lower, dim - 1 + upper].
+static int make_im2col_maps(TcMaps& maps, int i, const TcSubProblem& s, const TcWorkspace& ws, const TcConvCall& call, int BK) {
+    const int H = call.res_in;
+    const int lw = s.base_dx, lh = s.base_dy, uw = s.base_dx + s.ow - H, uh = s.base_dy + s.oh - H;
+    SIS_PROPAGATE(make_im2col_map(&maps.a[i][0], ws.a_hi[call.in_slot], call.cin, H, H, call.batch, lw, lh, uw, uh, BK, BK * 2));
+    SIS_PROPAGATE(make_im2col_map(&maps.a[i][1], ws.a_lo[call.in_slot], call.cin, H, H, call.batch, lw, lh, uw, uh, BK, BK * 2));
+    return SIS_OK;
+}
+
+// Taps of the plain 3x3 conv: tap t = ky*3 + kx reads the input at offset (ky - 1, kx - 1).
+static void set_conv_taps(TcSubProblem& s) {
+    s.ntaps = 9;
+    for (int ky = 0; ky < 3; ++ky)
+        for (int kx = 0; kx < 3; ++kx) { const int t = ky * 3 + kx; s.dy[t] = (short)(ky - 1); s.dx[t] = (short)(kx - 1); s.widx[t] = (signed char)t; }
+}
+
+// Appends the taps of output phase (py, px) of the stride-2 transposed conv.  F.conv_transpose2d(stride 2, pad 0),
+// model.py:259: out[2i+k] += x[i]*W[k], so phase p = o mod 2 takes the taps ky = py, kx = px (mod 2) at input offset
+// (-ky/2, -kx/2), shifted by the sub-problem's origin (y0, x0) when it starts inside the grid (the border strips).
+static void add_phase_taps(TcSubProblem& s, int py, int px, int y0 = 0, int x0 = 0) {
+    for (int ky = py; ky < 3; ky += 2)
+        for (int kx = px; kx < 3; kx += 2) {
+            s.dy[s.ntaps] = (short)(y0 - ky / 2); s.dx[s.ntaps] = (short)(x0 - kx / 2);
+            s.widx[s.ntaps] = (signed char)(ky * 3 + kx); s.phase[s.ntaps] = (signed char)(py * 2 + px); s.ntaps++;
+        }
+}
+
+// im2col runs of a per-tap sub-problem: 128 flattened output pixels each; the traversal box starts at the smallest tap offset.
+static void set_im2col_runs(TcSubProblem& s, int batch) {
+    s.m_tiles = (int)ceil_div64((int64_t)batch * s.oh * s.ow, BM);
+    s.base_dy = s.dy[0]; s.base_dx = s.dx[0];
+    for (int t = 1; t < s.ntaps; ++t) { s.base_dy = std::min<int>(s.base_dy, s.dy[t]); s.base_dx = std::min<int>(s.base_dx, s.dx[t]); }
+}
+
+// Arguments shared by the launches of one conv call.  Plain layers (mode 0) write the capture and the next conv's planes;
+// up-convs (mode 1) write the demodulated phases to the fp32 NHWC scratch that the blur pass reads.
+static TcKernelArgs conv_args(const TcWorkspace& ws, const TcConvCall& call, int BK) {
+    TcKernelArgs a;
+    memset(&a, 0, sizeof(a));
+    const int H = call.res_in;
+    a.batch = call.batch; a.cin = call.cin; a.cout = call.cout; a.kchunks = call.cin / BK; a.b_tiles = call.batch;
+    a.demod = call.demod; a.error = ws.d_error;
+    if (call.up) {
+        a.mode = 1;
+        a.out_f32 = call.upconv_tmp; a.out_h = 2 * H + 1; a.out_w = 2 * H + 1;
+    } else {
+        a.mode = 0; a.act = call.act ? 1 : 0;
+        a.noise = call.noise; a.noise_bstride = call.noise_bstride; a.noise_w = call.noise_w; a.bias = call.bias;
+        a.out_f32 = call.out_f32; a.out_h = H; a.out_w = H;
+        a.s_next = call.s_next; a.next_hi = (bf16*)ws.a_hi[call.out_slot]; a.next_lo = (bf16*)ws.a_lo[call.out_slot];
+    }
+    return a;
+}
+
+// Persistent launch of a GEMM kernel: one CTA (CG = 1) or CTA pair (CG = 2) per SM (pair), at most one per tile;
+// a.total_tiles counts tiles resp. pair tiles.
+template <auto Kernel, int SMEM_BYTES, int CG = 1>
+static int launch_persistent(const TcMaps& maps, const TcKernelArgs& a, cudaStream_t stream) {
     static bool configured = false;
     if (!configured) {
-        SIS_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
+        SIS_CHECK_CUDA(cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
         configured = true;
     }
-    // persistent: one CTA (CG = 1) or one CTA pair (CG = 2) per SM (pair); a.total_tiles counts tiles resp. pair tiles
-    int grid = a.total_tiles * CG < kNumSMs ? a.total_tiles * CG : kNumSMs;
-    const int st_used = a.stages > 0 && a.stages < Cfg::STAGES ? a.stages : Cfg::STAGES;
-    const size_t SMEM_USED = (size_t)st_used * Cfg::STAGE_BYTES + 1024 + 256;
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3(grid); cfg.blockDim = dim3(tc_threads()); cfg.dynamicSmemBytes = SMEM_USED; cfg.stream = stream;
+    cfg.gridDim = dim3(a.total_tiles * CG < kNumSMs ? a.total_tiles * CG : kNumSMs);
+    cfg.blockDim = dim3(TC_THREADS); cfg.dynamicSmemBytes = SMEM_BYTES; cfg.stream = stream;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
     attr[0].val.clusterDim.x = CG; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr; cfg.numAttrs = 1;
-    SIS_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, maps, a));
+    SIS_CHECK_CUDA(cudaLaunchKernelEx(&cfg, Kernel, maps, a));
     SIS_CHECK_LAUNCH();
     return SIS_OK;
 }
 
-template <int BN, int CG, int BK, bool UP4>
-static int launch_tc_halo(const TcMaps& maps, const TcKernelArgs& a, cudaStream_t stream) {
-    using Cfg = TcHaloCfg<BN, CG, BK, UP4>;
-    auto kern = modconv_tc_halo_kernel<BN, CG, BK, UP4>;
-    static bool configured = false;
-    if (!configured) {
-        SIS_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
-        configured = true;
+// Per-tap kernel by N tile.  CTA pairs are only chosen with BN >= 64 (each CTA's half of the weight tile must be a legal
+// UMMA N), so BN = 32 exists for single CTAs only.
+template <int BK, int CG>
+static int launch_tc(int BN, const TcMaps& maps, const TcKernelArgs& a, cudaStream_t stream) {
+    if (BN == 256) return launch_persistent<modconv_tc_kernel<256, BK, CG>, TcCfg<256, BK, CG>::SMEM_BYTES, CG>(maps, a, stream);
+    if (BN == 128) return launch_persistent<modconv_tc_kernel<128, BK, CG>, TcCfg<128, BK, CG>::SMEM_BYTES, CG>(maps, a, stream);
+    if (BN == 64) return launch_persistent<modconv_tc_kernel<64, BK, CG>, TcCfg<64, BK, CG>::SMEM_BYTES, CG>(maps, a, stream);
+    if constexpr (CG == 1) {
+        if (BN == 32) return launch_persistent<modconv_tc_kernel<32, BK, 1>, TcCfg<32, BK, 1>::SMEM_BYTES>(maps, a, stream);
     }
-    int grid = a.total_tiles * CG < kNumSMs ? a.total_tiles * CG : kNumSMs;
-    const int nb_used = a.stages > 0 && a.stages < Cfg::NB ? a.stages : Cfg::NB;
-    const size_t SMEM_USED = (size_t)Cfg::NA * Cfg::A_STAGE + (size_t)nb_used * Cfg::B_STAGE + 1024 + 512;
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3(grid); cfg.blockDim = dim3(tc_threads()); cfg.dynamicSmemBytes = SMEM_USED; cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = CG; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    SIS_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, maps, a));
-    SIS_CHECK_LAUNCH();
-    return SIS_OK;
-}
-
-template <int BN, int BK, bool UP4>
-static int launch_tc_halo_rw(const TcMaps& maps, const TcKernelArgs& a, cudaStream_t stream) {
-    using Cfg = TcHaloRwCfg<BN, BK, UP4>;
-    auto kern = modconv_tc_halo_rw_kernel<BN, BK, UP4>;
-    static bool configured = false;
-    if (!configured) {
-        SIS_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
-        configured = true;
-    }
-    const int grid = a.total_tiles < kNumSMs ? a.total_tiles : kNumSMs;
-    kern<<<grid, tc_threads(), Cfg::SMEM_BYTES, stream>>>(maps, a);
-    SIS_CHECK_LAUNCH();
-    return SIS_OK;
-}
-
-static int launch_tc_halo_t(const TcMaps& maps, const TcKernelArgs& a, cudaStream_t stream) {
-    using Cfg = TcHaloTCfg;
-    static bool configured = false;
-    if (!configured) {
-        SIS_CHECK_CUDA(cudaFuncSetAttribute(modconv_tc_halo_t_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
-        configured = true;
-    }
-    const int grid = a.total_tiles < kNumSMs ? a.total_tiles : kNumSMs;
-    modconv_tc_halo_t_kernel<<<grid, tc_threads(), Cfg::SMEM_BYTES, stream>>>(maps, a);
-    SIS_CHECK_LAUNCH();
-    return SIS_OK;
-}
-
-template <int CG>
-static int launch_tc_halo_any(int BN, int BK, const TcMaps& maps, const TcKernelArgs& a, cudaStream_t stream) {
-    if (BK == 32) {          // 32-channel K chunks are only built for the narrow layers that have them
-        if (BN == 64) return launch_tc_halo<64, CG, 32, false>(maps, a, stream);
-        return launch_tc_halo<32, CG, 32, false>(maps, a, stream);
-    }
-    if (BN == 256) return launch_tc_halo<256, CG, 64, false>(maps, a, stream);
-    if (BN == 128) return launch_tc_halo<128, CG, 64, false>(maps, a, stream);
-    if (BN == 64) return launch_tc_halo<64, CG, 64, false>(maps, a, stream);
-    return launch_tc_halo<32, CG, 64, false>(maps, a, stream);
-}
-
-// 4-phase halo kernel of the transposed conv with Cout <= 64 (BN = Cout)
-static int launch_tc_halo_up4(int BN, int BK, int CG, const TcMaps& maps, const TcKernelArgs& a, cudaStream_t stream) {
-    if (BN == 64) {
-        if (CG == 2) return BK == 64 ? launch_tc_halo<64, 2, 64, true>(maps, a, stream) : launch_tc_halo<64, 2, 32, true>(maps, a, stream);
-        return BK == 64 ? launch_tc_halo<64, 1, 64, true>(maps, a, stream) : launch_tc_halo<64, 1, 32, true>(maps, a, stream);
-    }
-    return BK == 64 ? launch_tc_halo<32, 1, 64, true>(maps, a, stream) : launch_tc_halo<32, 1, 32, true>(maps, a, stream);
-}
-
-template <int BN, int BK, int CG>
-static int launch_tc_bn(int th, int tw, int tb, const TcMaps& maps, const TcKernelArgs& a, cudaStream_t stream) {
-    if (th == 4 && tw == 4 && tb == 8) return launch_tc<BN, 4, 4, 8, BK, CG>(maps, a, stream);
-    if (th == 8 && tw == 8 && tb == 2) return launch_tc<BN, 8, 8, 2, BK, CG>(maps, a, stream);
-    if (th == 8 && tw == 16 && tb == 1) return launch_tc<BN, 8, 16, 1, BK, CG>(maps, a, stream);
-    set_error("tc_modconv: unsupported tile box %dx%dx%d", th, tw, tb);
+    set_error("tc_modconv: no per-tap kernel for BN %d with CG %d", BN, CG);
     return SIS_ERR_UNSUPPORTED;
 }
 
-template <int BK, int CG>
-static int launch_tc_any(int BN, int th, int tw, int tb, const TcMaps& maps, const TcKernelArgs& a, cudaStream_t stream) {
-    if (BN == 256) return launch_tc_bn<256, BK, CG>(th, tw, tb, maps, a, stream);
-    if (BN == 128) return launch_tc_bn<128, BK, CG>(th, tw, tb, maps, a, stream);
-    if (BN == 64) return launch_tc_bn<64, BK, CG>(th, tw, tb, maps, a, stream);
-    return launch_tc_bn<32, BK, CG>(th, tw, tb, maps, a, stream);
+// Halo kernel of the plain conv by N tile and K chunk (32-channel K chunks only for the narrow layers that have them).
+template <int CG>
+static int launch_tc_halo(int BN, int BK, const TcMaps& maps, const TcKernelArgs& a, cudaStream_t stream) {
+    if (BK == 32) {
+        if (BN == 64) return launch_persistent<modconv_tc_halo_kernel<64, CG, 32, false>, TcHaloCfg<64, CG, 32, false>::SMEM_BYTES, CG>(maps, a, stream);
+        if constexpr (CG == 1) {
+            if (BN == 32) return launch_persistent<modconv_tc_halo_kernel<32, 1, 32, false>, TcHaloCfg<32, 1, 32, false>::SMEM_BYTES>(maps, a, stream);
+        }
+    } else {
+        if (BN == 256) return launch_persistent<modconv_tc_halo_kernel<256, CG, 64, false>, TcHaloCfg<256, CG, 64, false>::SMEM_BYTES, CG>(maps, a, stream);
+        if (BN == 128) return launch_persistent<modconv_tc_halo_kernel<128, CG, 64, false>, TcHaloCfg<128, CG, 64, false>::SMEM_BYTES, CG>(maps, a, stream);
+        if (BN == 64) return launch_persistent<modconv_tc_halo_kernel<64, CG, 64, false>, TcHaloCfg<64, CG, 64, false>::SMEM_BYTES, CG>(maps, a, stream);
+        if constexpr (CG == 1) {
+            if (BN == 32) return launch_persistent<modconv_tc_halo_kernel<32, 1, 64, false>, TcHaloCfg<32, 1, 64, false>::SMEM_BYTES>(maps, a, stream);
+        }
+    }
+    set_error("tc_modconv: no halo kernel for BN %d, BK %d with CG %d", BN, BK, CG);
+    return SIS_ERR_UNSUPPORTED;
+}
+
+// 4-phase halo kernel of the transposed conv with Cout <= 64 (BN = Cout; CTA pairs for BN = 64 only)
+static int launch_tc_halo_up4(int BN, int BK, int CG, const TcMaps& maps, const TcKernelArgs& a, cudaStream_t stream) {
+    if (BN == 64 && CG == 2) {
+        if (BK == 64) return launch_persistent<modconv_tc_halo_kernel<64, 2, 64, true>, TcHaloCfg<64, 2, 64, true>::SMEM_BYTES, 2>(maps, a, stream);
+        return launch_persistent<modconv_tc_halo_kernel<64, 2, 32, true>, TcHaloCfg<64, 2, 32, true>::SMEM_BYTES, 2>(maps, a, stream);
+    }
+    if (BN == 64) {
+        if (BK == 64) return launch_persistent<modconv_tc_halo_kernel<64, 1, 64, true>, TcHaloCfg<64, 1, 64, true>::SMEM_BYTES>(maps, a, stream);
+        return launch_persistent<modconv_tc_halo_kernel<64, 1, 32, true>, TcHaloCfg<64, 1, 32, true>::SMEM_BYTES>(maps, a, stream);
+    }
+    if (BK == 64) return launch_persistent<modconv_tc_halo_kernel<32, 1, 64, true>, TcHaloCfg<32, 1, 64, true>::SMEM_BYTES>(maps, a, stream);
+    return launch_persistent<modconv_tc_halo_kernel<32, 1, 32, true>, TcHaloCfg<32, 1, 32, true>::SMEM_BYTES>(maps, a, stream);
 }
 
 // Second half of an up-sampling layer: Blur(4x4, pad 1) + noise + bias + lrelu over the fp32 NHWC scratch.
 template <int CB>
-static int launch_blur_split(const BlurSplitArgs& bs, int ring, bool sep, cudaStream_t stream) {
+static int launch_blur_split(const BlurSplitArgs& bs, bool sep, cudaStream_t stream) {
     using G = BlurGeo<CB>;
-    if (CB != 64 && ring == 0) ring = 2;                   // cp.async staging exists for 64-channel blocks only
-    static int blocks_per_sm[6] = {0, 0, 0, 0, 0, 0};
-    const int variant = (sep ? 1 : 0) + 2 * ring;
-    const size_t smem = ring == 2 ? 2 * (size_t)G::SMEM + 128 : ring == 1 ? (size_t)G::SMEM + 128 : (size_t)G::SMEM;
-    void (*kern)(BlurSplitArgs, const CUtensorMap);
-    if (CB == 64 && ring == 0) kern = sep ? blur_act_split_kernel<true, 0, 64> : blur_act_split_kernel<false, 0, 64>;
-    else if (ring == 1) kern = sep ? blur_act_split_kernel<true, 1, CB> : blur_act_split_kernel<false, 1, CB>;
-    else kern = sep ? blur_act_split_kernel<true, 2, CB> : blur_act_split_kernel<false, 2, CB>;
-    if (!blocks_per_sm[variant]) {
+    static int blocks_per_sm[2] = {0, 0};                  // by `sep`
+    const size_t smem = 2 * (size_t)G::SMEM + 128;         // the ring of two input tiles + alignment
+    auto kern = sep ? blur_act_split_kernel<true, CB> : blur_act_split_kernel<false, CB>;
+    int& bps = blocks_per_sm[sep ? 1 : 0];
+    if (!bps) {
         SIS_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        SIS_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm[variant], kern, 256, smem));
-        if (blocks_per_sm[variant] < 1) blocks_per_sm[variant] = 1;
+        SIS_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, kern, 256, smem));
+        if (bps < 1) bps = 1;
     }
     CUtensorMap in_map;
     memset(&in_map, 0, sizeof(in_map));
-    if (ring > 0) {
-        const uint64_t dims[4] = {(uint64_t)bs.C, (uint64_t)bs.IW, (uint64_t)bs.IH, (uint64_t)bs.batch};
-        const uint32_t box[4] = {(uint32_t)CB, (uint32_t)G::IW, (uint32_t)BS_IH, 1};
-        SIS_PROPAGATE(make_map_f32(&in_map, bs.in, 4, dims, box));
-    }
+    const uint64_t dims[4] = {(uint64_t)bs.C, (uint64_t)bs.IW, (uint64_t)bs.IH, (uint64_t)bs.batch};
+    const uint32_t box[4] = {(uint32_t)CB, (uint32_t)G::IW, (uint32_t)BS_IH, 1};
+    SIS_PROPAGATE(make_map_f32(&in_map, bs.in, 4, dims, box));
     const int64_t total = (int64_t)bs.batch * ceil_div(bs.OH, BS_TH) * ceil_div(bs.OW, G::TW) * ceil_div(bs.C, CB);
-    const int grid = (int)std::min<int64_t>(total, (int64_t)kNumSMs * blocks_per_sm[variant]);   // exactly one resident wave
+    const int grid = (int)std::min<int64_t>(total, (int64_t)kNumSMs * bps);   // exactly one resident wave
     ProfScope prof(PROF_BLUR_SPLIT, stream);
     kern<<<grid, 256, smem, stream>>>(bs, in_map);
     SIS_CHECK_LAUNCH();
@@ -1839,106 +1804,54 @@ static int tc_blur_after_upconv(TcWorkspace& ws, const TcConvCall& call, cudaStr
     bs.s_next = call.s_next; bs.next_hi = (bf16*)ws.a_hi[call.out_slot]; bs.next_lo = (bf16*)ws.a_lo[call.out_slot];
     bs.act = call.act ? 1 : 0;
     SIS_REQUIRE(bs.C % 32 == 0, "tc_modconv: the blur pass needs Cout %% 32 == 0 (got %d)", bs.C);
-    static int ring_env = env_int("SIS_BLUR_TMA", 2);      // 0: cp.async, 1: TMA single buffer (3 blocks/SM), 2: TMA ring of 2
-    const int ring = (bs.C * 4) % 16 == 0 ? (ring_env < 0 ? 0 : ring_env > 2 ? 2 : ring_env) : 0;
     // 32-channel blocks when the channel count is an odd multiple of 32 (the 1024^2 layer): no idle lanes
-    if (bs.C % 64 != 0 && bs.OW >= 32) return launch_blur_split<32>(bs, ring, call.blur_separable, stream);
-    return launch_blur_split<64>(bs, ring, call.blur_separable, stream);
+    if (bs.C % 64 != 0 && bs.OW >= 32) return launch_blur_split<32>(bs, call.blur_separable, stream);
+    return launch_blur_split<64>(bs, call.blur_separable, stream);
 }
 
 int tc_modconv(TcWorkspace& ws, const TcConvWeights& w, const TcConvCall& call, cudaStream_t stream) {
     // layers with Cout <= 64 are timed apart: SURVEY §8(d)'s ridge check reports them against HBM, not the tensor peak
     const int conv_cat = call.cout <= 64 ? PROF_CONV_TC_NARROW : PROF_CONV_TC;
-    // Tunables for A/B runs: SIS_TC_BK (64 default | 32: stage depth along K), SIS_TC_CG (2 default | 1: CTA pairs)
-    //                       SIS_TC_IM2COL (1 default | 0: spatial-box A tiles instead of flattened 128-pixel runs)
-    //                       SIS_TC_HALO (1 default | 0: per-tap A tiles on the plain layers too)
-    static int bk_env = 0, cg_env = 0, im2col_env = 1, halo_env = 1;
-    if (!bk_env) {
-        bk_env = env_int("SIS_TC_BK", 64) == 32 ? 32 : 64; cg_env = env_int("SIS_TC_CG", 2) == 1 ? 1 : 2;
-        im2col_env = env_int("SIS_TC_IM2COL", 1) != 0;
-        halo_env = env_int("SIS_TC_HALO", 1) != 0;
-    }
-    // transposed halo kernel: Cout = 128 plain layers that feed no further conv (SIS_TC_TRANSPOSED=0 disables)
-    static int transposed_env = env_int("SIS_TC_TRANSPOSED", 1);
-    if (transposed_env && halo_env && !call.up && call.cout == 128 && call.cin % HT_BK == 0 && call.res_in % HT_TH == 0) {
-        SIS_REQUIRE(w.hi && w.cin == call.cin && w.cout == call.cout, "tc_modconv: weights not packed for this layer");
-        TcKernelArgs a;
-        memset(&a, 0, sizeof(a));
-        const int H = call.res_in;
-        a.batch = call.batch; a.cin = call.cin; a.cout = call.cout; a.kchunks = call.cin / HT_BK;
-        a.b_tiles = call.batch; a.n_tiles = call.cout / 128;
-        a.demod = call.demod; a.noise = call.noise; a.noise_bstride = call.noise_bstride; a.noise_w = call.noise_w; a.bias = call.bias;
-        a.error = ws.d_error; a.act = call.act ? 1 : 0; a.mode = 0; a.nsub = 1;
+    SIS_REQUIRE(w.hi && w.cin == call.cin && w.cout == call.cout, "tc_modconv: weights not packed for this layer");
+    const int B = call.batch, H = call.res_in;
+    // transposed halo kernel: Cout = 128 plain layers whose image holds whole 32 x 8 tiles
+    if (!call.up && call.cout == 128 && call.cin % HT_BK == 0 && H % HT_TH == 0) {
+        TcKernelArgs a = conv_args(ws, call, HT_BK);
+        a.nsub = 1;
         TcSubProblem& s = a.sub[0];
-        s.ntaps = 9;
-        for (int ky = 0; ky < 3; ++ky)
-            for (int kx = 0; kx < 3; ++kx) { int t = ky * 3 + kx; s.dy[t] = (short)(ky - 1); s.dx[t] = (short)(kx - 1); s.widx[t] = (signed char)t; }
+        set_conv_taps(s);
         s.oh = H; s.ow = H; s.ostride = 1;
-        a.total_tiles = call.batch * (H / HT_TH) * (H / HT_TW) * a.n_tiles;
-        a.out_f32 = call.out_f32; a.out_h = H; a.out_w = H;
-        a.s_next = call.s_next; a.next_hi = (bf16*)ws.a_hi[call.out_slot]; a.next_lo = (bf16*)ws.a_lo[call.out_slot];
+        a.total_tiles = B * (H / HT_TH) * (H / HT_TW);
         TcMaps maps;
         memset(&maps, 0, sizeof(maps));
-        const uint64_t adims[4] = {(uint64_t)call.cin, (uint64_t)H, (uint64_t)H, (uint64_t)call.batch};
-        const uint32_t abox[4] = {(uint32_t)HT_BK, (uint32_t)HT_W, (uint32_t)HT_H, 1};
-        SIS_PROPAGATE(make_map(&maps.a[0][0], ws.a_hi[call.in_slot], 4, adims, abox, HT_BK * 2));
-        SIS_PROPAGATE(make_map(&maps.a[0][1], ws.a_lo[call.in_slot], 4, adims, abox, HT_BK * 2));
-        const uint64_t wdims[3] = {(uint64_t)call.cin, (uint64_t)call.cout, 9};
-        const uint32_t wbox[3] = {(uint32_t)HT_BK, 128, 1};
-        SIS_PROPAGATE(make_map(&maps.w[0], w.hi, 3, wdims, wbox, HT_BK * 2));
-        SIS_PROPAGATE(make_map(&maps.w[1], w.lo, 3, wdims, wbox, HT_BK * 2));
+        SIS_PROPAGATE(make_halo_maps(maps, ws, call, HT_BK, HT_W, HT_H));
+        SIS_PROPAGATE(make_weight_maps(maps, w.hi, w.lo, call.cin, call.cout, 9, HT_BK, 128));
         ProfScope prof(conv_cat, stream);
-        return launch_tc_halo_t(maps, a, stream);
+        return launch_persistent<modconv_tc_halo_t_kernel, TcHaloTCfg::SMEM_BYTES>(maps, a, stream);
     }
     // Cout = 128 up-convs: the interior H x H of the four phase grids on the transposed halo kernel (exact 32 x 8 tiles),
-    // the one extra row / column of the (H+1)-extent phases as four thin strips on the per-tap kernel below
-    static int up_t_env = env_int("SIS_TC_UP_T", 1) != 0;
-    const bool up_split = transposed_env && halo_env && im2col_env && call.up && call.cout == 128 && call.cin % 64 == 0 &&
-                          call.res_in % HT_TH == 0 && call.res_in <= 128 /* im2col box corners are 8-bit */ && up_t_env;
-    if (up_split) {
-        SIS_REQUIRE(w.hi && w.cin == call.cin && w.cout == call.cout, "tc_modconv: weights not packed for this layer");
-        TcKernelArgs a;
-        memset(&a, 0, sizeof(a));
-        const int H = call.res_in;
-        a.batch = call.batch; a.cin = call.cin; a.cout = call.cout; a.kchunks = call.cin / HT_BK;
-        a.b_tiles = call.batch; a.n_tiles = 1;
-        a.demod = call.demod; a.error = ws.d_error; a.mode = 1; a.nsub = 4;
-        int si = 0;
-        for (int py = 0; py < 2; ++py)
-            for (int px = 0; px < 2; ++px) {
-                TcSubProblem& s = a.sub[si++];
-                s.ntaps = 0;
-                for (int ky = py; ky < 3; ky += 2)
-                    for (int kx = px; kx < 3; kx += 2) {
-                        s.dy[s.ntaps] = (short)(-(ky / 2)); s.dx[s.ntaps] = (short)(-(kx / 2));
-                        s.widx[s.ntaps] = (signed char)(ky * 3 + kx); s.ntaps++;
-                    }
-                s.oh = H; s.ow = H; s.ostride = 2; s.ooff_y = py; s.ooff_x = px;
-            }
-        a.total_tiles = call.batch * (H / HT_TH) * (H / HT_TW) * 4;
-        a.out_f32 = call.upconv_tmp; a.out_h = 2 * H + 1; a.out_w = 2 * H + 1;
+    // the one extra row / column of the (H+1)-extent phases as four thin strips on the per-tap kernel
+    if (call.up && call.cout == 128 && call.cin % 64 == 0 && H % HT_TH == 0 && H <= 128 /* im2col box corners are 8-bit */) {
+        TcKernelArgs a = conv_args(ws, call, HT_BK);
+        a.nsub = 4;
+        for (int p = 0; p < 4; ++p) {
+            TcSubProblem& s = a.sub[p];
+            add_phase_taps(s, p >> 1, p & 1);
+            s.oh = H; s.ow = H; s.ostride = 2; s.ooff_y = p >> 1; s.ooff_x = p & 1;
+        }
+        a.total_tiles = B * (H / HT_TH) * (H / HT_TW) * 4;
         TcMaps maps;
         memset(&maps, 0, sizeof(maps));
-        const uint64_t adims[4] = {(uint64_t)call.cin, (uint64_t)H, (uint64_t)H, (uint64_t)call.batch};
-        const uint32_t abox[4] = {(uint32_t)HT_BK, (uint32_t)HT_W, (uint32_t)HT_H, 1};
-        SIS_PROPAGATE(make_map(&maps.a[0][0], ws.a_hi[call.in_slot], 4, adims, abox, HT_BK * 2));
-        SIS_PROPAGATE(make_map(&maps.a[0][1], ws.a_lo[call.in_slot], 4, adims, abox, HT_BK * 2));
-        const uint64_t wdims[3] = {(uint64_t)call.cin, (uint64_t)call.cout, 9};
-        const uint32_t wbox[3] = {(uint32_t)HT_BK, 128, 1};
-        SIS_PROPAGATE(make_map(&maps.w[0], w.hi, 3, wdims, wbox, HT_BK * 2));
-        SIS_PROPAGATE(make_map(&maps.w[1], w.lo, 3, wdims, wbox, HT_BK * 2));
+        SIS_PROPAGATE(make_halo_maps(maps, ws, call, HT_BK, HT_W, HT_H));
+        SIS_PROPAGATE(make_weight_maps(maps, w.hi, w.lo, call.cin, call.cout, 9, HT_BK, 128));
         {
             ProfScope prof(conv_cat, stream);
-            SIS_PROPAGATE(launch_tc_halo_t(maps, a, stream));
+            SIS_PROPAGATE((launch_persistent<modconv_tc_halo_t_kernel, TcHaloTCfg::SMEM_BYTES>(maps, a, stream)));
         }
         // strips: (py=0) row yy = H of phases (0,0) [xx 0..H] and (0,1) [xx 0..H-1]; (px=0) column xx = H of phases
         // (0,0) and (1,0) [yy 0..H-1].  Origins are folded into the tap offsets and the output offsets.
-        TcKernelArgs b;
-        memset(&b, 0, sizeof(b));
-        b.batch = call.batch; b.cin = call.cin; b.cout = call.cout; b.kchunks = call.cin / 64;
-        b.b_tiles = call.batch; b.n_tiles = 1;
-        b.demod = call.demod; b.error = ws.d_error; b.mode = 1; b.im2col = 1; b.nsub = 4;
-        b.out_f32 = call.upconv_tmp; b.out_h = 2 * H + 1; b.out_w = 2 * H + 1;
+        TcKernelArgs b = conv_args(ws, call, 64);
+        b.nsub = 4;
         struct Strip { int py, px, y0, x0, oh, ow; };
         const Strip strips[4] = {{0, 0, H, 0, 1, H + 1}, {0, 1, H, 0, 1, H}, {0, 0, 0, H, H, 1}, {1, 0, 0, H, H, 1}};
         TcMaps mb;
@@ -1947,100 +1860,58 @@ int tc_modconv(TcWorkspace& ws, const TcConvWeights& w, const TcConvCall& call, 
         for (int i = 0; i < 4; ++i) {
             const Strip& sp = strips[i];
             TcSubProblem& s = b.sub[i];
-            s.ntaps = 0;
-            for (int ky = sp.py; ky < 3; ky += 2)
-                for (int kx = sp.px; kx < 3; kx += 2) {
-                    s.dy[s.ntaps] = (short)(sp.y0 - ky / 2); s.dx[s.ntaps] = (short)(sp.x0 - kx / 2);
-                    s.widx[s.ntaps] = (signed char)(ky * 3 + kx); s.ntaps++;
-                }
+            add_phase_taps(s, sp.py, sp.px, sp.y0, sp.x0);
             s.oh = sp.oh; s.ow = sp.ow; s.ostride = 2; s.ooff_y = 2 * sp.y0 + sp.py; s.ooff_x = 2 * sp.x0 + sp.px;
-            s.m_tiles = (int)ceil_div64((int64_t)call.batch * s.oh * s.ow, BM);
-            s.base_dy = 32767; s.base_dx = 32767;
-            for (int t = 0; t < s.ntaps; ++t) { s.base_dy = std::min<int>(s.base_dy, s.dy[t]); s.base_dx = std::min<int>(s.base_dx, s.dx[t]); }
-            s.tiles_y = 1; s.tiles_x = 1; s.tile_begin = tiles;
+            set_im2col_runs(s, B);
+            s.tile_begin = tiles;
             tiles += s.m_tiles;
-            const int lw = s.base_dx, lh = s.base_dy, uw = s.base_dx + s.ow - H, uh = s.base_dy + s.oh - H;
-            SIS_PROPAGATE(make_im2col_map(&mb.a[i][0], ws.a_hi[call.in_slot], call.cin, H, H, call.batch, lw, lh, uw, uh, 64, 128));
-            SIS_PROPAGATE(make_im2col_map(&mb.a[i][1], ws.a_lo[call.in_slot], call.cin, H, H, call.batch, lw, lh, uw, uh, 64, 128));
+            SIS_PROPAGATE(make_im2col_maps(mb, i, s, ws, call, 64));
         }
         b.total_tiles = tiles;
-        const uint32_t wbox64[3] = {64, 128, 1};
-        SIS_PROPAGATE(make_map(&mb.w[0], w.hi, 3, wdims, wbox64, 128));
-        SIS_PROPAGATE(make_map(&mb.w[1], w.lo, 3, wdims, wbox64, 128));
+        SIS_PROPAGATE(make_weight_maps(mb, w.hi, w.lo, call.cin, call.cout, 9, 64, 128));
         {
             ProfScope prof(conv_cat, stream);
-            SIS_PROPAGATE((launch_tc<128, 8, 16, 1, 64, 1>(mb, b, stream)));
+            SIS_PROPAGATE((launch_tc<64, 1>(128, mb, b, stream)));
         }
         return tc_blur_after_upconv(ws, call, stream);
     }
     // Cout <= 64 up-convs (the 512^2 / 1024^2 models): all four output phases of a spatial tile from ONE halo per K chunk
-    static int up4_env = env_int("SIS_TC_UP4", 1) != 0;
-    if (up4_env && halo_env && call.up && (call.cout == 64 || call.cout == 32) && call.cin % 32 == 0 && call.res_in >= 8) {
-        SIS_REQUIRE(w.hi && w.cin == call.cin && w.cout == call.cout, "tc_modconv: weights not packed for this layer");
-        const int B = call.batch, H = call.res_in, BN = call.cout, BK = call.cin % 64 == 0 ? 64 : 32;
-        TcKernelArgs a;
-        memset(&a, 0, sizeof(a));
-        a.batch = B; a.cin = call.cin; a.cout = call.cout; a.kchunks = call.cin / BK;
-        a.b_tiles = B; a.n_tiles = 1;
-        a.demod = call.demod; a.error = ws.d_error; a.mode = 1; a.nsub = 1;
+    if (call.up && (call.cout == 64 || call.cout == 32) && call.cin % 32 == 0 && H >= 8) {
+        const int BN = call.cout, BK = call.cin % 64 == 0 ? 64 : 32;
+        TcKernelArgs a = conv_args(ws, call, BK);
+        a.nsub = 1;
         TcSubProblem& s = a.sub[0];
-        s.ntaps = 0;
-        for (int py = 0; py < 2; ++py)
-            for (int px = 0; px < 2; ++px)
-                for (int ky = py; ky < 3; ky += 2)
-                    for (int kx = px; kx < 3; kx += 2) {
-                        s.dy[s.ntaps] = (short)(-(ky / 2)); s.dx[s.ntaps] = (short)(-(kx / 2));
-                        s.widx[s.ntaps] = (signed char)(ky * 3 + kx); s.phase[s.ntaps] = (signed char)(py * 2 + px); s.ntaps++;
-                    }
+        for (int p = 0; p < 4; ++p) add_phase_taps(s, p >> 1, p & 1);
         // tiles cover the (H+1)^2 grid of the py = px = 0 phase; the other phases' last row / column is masked in the epilogue
-        s.oh = H + 1; s.ow = H + 1; s.ostride = 2; s.ooff_y = 0; s.ooff_x = 0;
-        s.tiles_y = ceil_div(H + 1, HALO_TH); s.tiles_x = ceil_div(H + 1, HALO_TW); s.tile_begin = 0;
+        s.oh = H + 1; s.ow = H + 1; s.ostride = 2;
+        s.tiles_y = ceil_div(H + 1, HALO_TH); s.tiles_x = ceil_div(H + 1, HALO_TW);
         const int64_t m_tiles = (int64_t)B * s.tiles_y * s.tiles_x;
-        const int CG = (cg_env == 2 && BN == 64 && m_tiles >= 2 * kNumSMs) ? 2 : 1;
-        // 64 -> 32: all nine weight tiles stay resident in shared memory (SIS_TC_RW=0 streams them per tap)
-        static int rw_env = env_int("SIS_TC_RW", 1) != 0;
-        const bool rw = rw_env && BN == 32 && BK == 64 && a.kchunks == 1;
+        const int CG = (BN == 64 && m_tiles >= 2 * kNumSMs) ? 2 : 1;
         a.total_tiles = (int)ceil_div64(m_tiles, CG);
-        a.out_f32 = call.upconv_tmp; a.out_h = 2 * H + 1; a.out_w = 2 * H + 1;
         TcMaps maps;
         memset(&maps, 0, sizeof(maps));
-        const uint64_t adims[4] = {(uint64_t)call.cin, (uint64_t)H, (uint64_t)H, (uint64_t)B};
-        const uint32_t abox[4] = {(uint32_t)BK, (uint32_t)HALO_W, (uint32_t)HALO_H, 1};
-        SIS_PROPAGATE(make_map(&maps.a[0][0], ws.a_hi[call.in_slot], 4, adims, abox, BK * 2));
-        SIS_PROPAGATE(make_map(&maps.a[0][1], ws.a_lo[call.in_slot], 4, adims, abox, BK * 2));
-        const uint64_t wdims[3] = {(uint64_t)call.cin, (uint64_t)call.cout, 9};
-        const uint32_t wbox[3] = {(uint32_t)BK, (uint32_t)(BN / CG), 1};
-        SIS_PROPAGATE(make_map(&maps.w[0], w.hi, 3, wdims, wbox, BK * 2));
-        SIS_PROPAGATE(make_map(&maps.w[1], w.lo, 3, wdims, wbox, BK * 2));
+        SIS_PROPAGATE(make_halo_maps(maps, ws, call, BK, HALO_W, HALO_H));
+        SIS_PROPAGATE(make_weight_maps(maps, w.hi, w.lo, call.cin, call.cout, 9, BK, BN / CG));
         {
             ProfScope prof(conv_cat, stream);
-            if (rw) SIS_PROPAGATE((launch_tc_halo_rw<32, 64, true>(maps, a, stream)));
-            else SIS_PROPAGATE(launch_tc_halo_up4(BN, BK, CG, maps, a, stream));
+            // 64 -> 32: all nine weight tiles stay resident in shared memory
+            if (BN == 32 && BK == 64 && a.kchunks == 1)
+                SIS_PROPAGATE((launch_persistent<modconv_tc_halo_rw_kernel<32, 64, true>, TcHaloRwCfg<32, 64, true>::SMEM_BYTES>(maps, a, stream)));
+            else
+                SIS_PROPAGATE(launch_tc_halo_up4(BN, BK, CG, maps, a, stream));
         }
         return tc_blur_after_upconv(ws, call, stream);
     }
     // halo reuse: plain 3x3 layers whose image holds whole 16 x 8 tiles; K chunks of 64 channels (128 B rows), or of 32
-    // (64 B rows) for the narrow layers with 32 input channels
-    const bool halo = halo_env && !call.up && call.res_in >= HALO_TH && call.res_in % HALO_TH == 0 &&
-                      (call.cin % 64 == 0 || (call.cin % 32 == 0 && call.cout <= 64));
-    const bool im2col = im2col_env != 0 && !halo;
-    const int BK = halo ? (call.cin % 64 == 0 ? 64 : 32) : (call.cin % 64 == 0) ? bk_env : 32;
+    // (64 B rows) for the narrow layers with 32 input channels.  Everything else runs on the per-tap kernel.
+    const bool halo = !call.up && H >= HALO_TH && H % HALO_TH == 0 && (call.cin % 64 == 0 || (call.cin % 32 == 0 && call.cout <= 64));
+    const int BK = call.cin % 64 == 0 ? 64 : 32;
     SIS_REQUIRE(call.cin % BK == 0, "tc_modconv: Cin must be a multiple of 32 (got %d)", call.cin);
     SIS_REQUIRE(call.cout % 32 == 0, "tc_modconv: Cout must be a multiple of 32 (got %d)", call.cout);
-    SIS_REQUIRE(w.hi && w.cin == call.cin && w.cout == call.cout, "tc_modconv: weights not packed for this layer");
-    const int B = call.batch, H = call.res_in;
-    // tile box by the GEMM grid extent (plain: H; transposed phases: up to H+1)
-    const int ext = call.up ? H + 1 : H;
-    int th, tw, tb;
-    if (halo) { th = HALO_TH; tw = HALO_TW; tb = 1; }
-    else if (im2col || ext > 8) { th = 8; tw = 16; tb = 1; }      // im2col mode ignores the box (one kernel variant)
-    else if (ext <= 4) { th = 4; tw = 4; tb = 8; }
-    else { th = 8; tw = 8; tb = 2; }
-    const int b_tiles = ceil_div(B, tb);
     // N tile: as wide as possible (fewest re-reads of the A tile) while the launch still fills the 148 SMs; the 4x4 and
     // 8x8 layers only have a handful of pixel tiles, so they run narrow N tiles on many CTAs instead of 8 fat ones
-    const int64_t m_tiles_all = im2col ? ceil_div64((int64_t)B * (call.up ? (2 * H + 1) * (2 * H + 1) : H * H), BM)
-                                       : (int64_t)b_tiles * ceil_div(ext, th) * ceil_div(ext, tw) * (call.up ? 4 : 1);
+    const int64_t m_tiles_all = halo ? (int64_t)B * ceil_div(H, HALO_TH) * ceil_div(H, HALO_TW)
+                                     : ceil_div64((int64_t)B * (call.up ? (2 * H + 1) * (2 * H + 1) : H * H), BM);
     int BN = 32;
     for (int cand = 256; cand >= 32; cand /= 2) {
         if (call.cout % cand) continue;
@@ -2065,100 +1936,55 @@ int tc_modconv(TcWorkspace& ws, const TcConvWeights& w, const TcConvCall& call, 
     SIS_REQUIRE(call.cout % BN == 0, "tc_modconv: unsupported Cout %d", call.cout);
     const int n_tiles = call.cout / BN;
     // CTA pairs only when there is at least one full wave of pair tiles and each CTA's weight half is a legal UMMA N
-    const int CG = (cg_env == 2 && BN >= 64 && m_tiles_all * n_tiles >= 2 * kNumSMs) ? 2 : 1;
+    const int CG = (BN >= 64 && m_tiles_all * n_tiles >= 2 * kNumSMs) ? 2 : 1;
 
-    TcKernelArgs a;
-    memset(&a, 0, sizeof(a));
-    a.batch = B; a.cin = call.cin; a.cout = call.cout; a.kchunks = call.cin / BK;
-    a.b_tiles = b_tiles; a.n_tiles = n_tiles;
-    a.demod = call.demod; a.noise = call.noise; a.noise_bstride = call.noise_bstride; a.noise_w = call.noise_w; a.bias = call.bias;
-    a.error = ws.d_error;
-    a.act = call.act ? 1 : 0;
-    static int stages_env = env_int("SIS_TC_STAGES", 0);      // experiment: cap the ring depth (0 = maximum)
-    a.stages = stages_env;
-    a.im2col = im2col ? 1 : 0;
-    int tiles = 0;   // tiles (CG = 1) or pair tiles (CG = 2)
-    auto units = [&](TcSubProblem& s) {
-        s.m_tiles = (int)ceil_div64((int64_t)B * s.oh * s.ow, BM);
-        s.base_dy = 127; s.base_dx = 127;
-        for (int t = 0; t < s.ntaps; ++t) { s.base_dy = std::min<int>(s.base_dy, s.dy[t]); s.base_dx = std::min<int>(s.base_dx, s.dx[t]); }
-        return ceil_div(im2col ? s.m_tiles : a.b_tiles * s.tiles_y * s.tiles_x, CG) * a.n_tiles;
-    };
+    TcKernelArgs a = conv_args(ws, call, BK);
     if (!call.up) {
-        a.mode = 0; a.nsub = 1;
+        a.nsub = 1;
         TcSubProblem& s = a.sub[0];
-        s.ntaps = 9;
-        for (int ky = 0; ky < 3; ++ky)
-            for (int kx = 0; kx < 3; ++kx) { int t = ky * 3 + kx; s.dy[t] = (short)(ky - 1); s.dx[t] = (short)(kx - 1); s.widx[t] = (signed char)t; }
-        s.oh = H; s.ow = H; s.ostride = 1; s.ooff_y = 0; s.ooff_x = 0;
-        s.tiles_y = ceil_div(H, th); s.tiles_x = ceil_div(H, tw); s.tile_begin = 0;
-        tiles = units(s);
-        a.out_f32 = call.out_f32; a.out_h = H; a.out_w = H;
-        a.s_next = call.s_next; a.next_hi = (bf16*)ws.a_hi[call.out_slot]; a.next_lo = (bf16*)ws.a_lo[call.out_slot];
-    } else {
-        // F.conv_transpose2d(stride 2, pad 0), model.py:259: out[2i+k] += x[i]*W[k]; phase p = o mod 2.
-        a.mode = 1; a.nsub = 4;
-        int si = 0;
-        for (int py = 0; py < 2; ++py)
-            for (int px = 0; px < 2; ++px) {
-                TcSubProblem& s = a.sub[si++];
-                s.ntaps = 0;
-                for (int ky = py; ky < 3; ky += 2)
-                    for (int kx = px; kx < 3; kx += 2) {
-                        s.dy[s.ntaps] = (short)(-(ky / 2)); s.dx[s.ntaps] = (short)(-(kx / 2));
-                        s.widx[s.ntaps] = (signed char)(ky * 3 + kx); s.ntaps++;
-                    }
-                s.oh = H + (py == 0 ? 1 : 0); s.ow = H + (px == 0 ? 1 : 0);
-                s.ostride = 2; s.ooff_y = py; s.ooff_x = px;
-                s.tiles_y = ceil_div(s.oh, th); s.tiles_x = ceil_div(s.ow, tw);
-                s.tile_begin = tiles;
-                tiles += units(s);
-            }
-        a.out_f32 = call.upconv_tmp; a.out_h = 2 * H + 1; a.out_w = 2 * H + 1;
-        static int il_env = -1;
-        if (il_env < 0) il_env = env_int("SIS_TC_INTERLEAVE", 1) != 0;
-        if (im2col && il_env) {
-            int umax = 0;
-            for (int i = 0; i < 4; ++i) umax = std::max(umax, ceil_div(a.sub[i].m_tiles, CG));
-            a.interleave_units = umax;
-            tiles = 4 * umax * a.n_tiles;
+        set_conv_taps(s);
+        s.oh = H; s.ow = H; s.ostride = 1;
+        if (halo) {
+            s.tiles_y = ceil_div(H, HALO_TH); s.tiles_x = ceil_div(H, HALO_TW);
+            a.total_tiles = ceil_div(B * s.tiles_y * s.tiles_x, CG) * n_tiles;
+        } else {
+            set_im2col_runs(s, B);
+            a.total_tiles = ceil_div(s.m_tiles, CG) * n_tiles;
         }
+    } else {
+        // the 4 phase sub-GEMMs walk the image together (see decode_tile), each padded to the largest one's (pair) tiles
+        a.nsub = 4;
+        int umax = 0;
+        for (int p = 0; p < 4; ++p) {
+            TcSubProblem& s = a.sub[p];
+            const int py = p >> 1, px = p & 1;
+            add_phase_taps(s, py, px);
+            s.oh = H + (py == 0 ? 1 : 0); s.ow = H + (px == 0 ? 1 : 0);
+            s.ostride = 2; s.ooff_y = py; s.ooff_x = px;
+            set_im2col_runs(s, B);
+            umax = std::max(umax, ceil_div(s.m_tiles, CG));
+        }
+        a.interleave_units = umax;
+        a.total_tiles = 4 * umax * n_tiles;
     }
-    a.total_tiles = tiles;
 
     TcMaps maps;
     memset(&maps, 0, sizeof(maps));
-    {
-        if (im2col) {
-            // traversal box of sub-problem s: base pixels [base_d, base_d + extent - 1] = [lower, dim - 1 + upper]
-            for (int i = 0; i < a.nsub; ++i) {
-                const TcSubProblem& s = a.sub[i];
-                const int lw = s.base_dx, lh = s.base_dy, uw = s.base_dx + s.ow - H, uh = s.base_dy + s.oh - H;
-                SIS_PROPAGATE(make_im2col_map(&maps.a[i][0], ws.a_hi[call.in_slot], call.cin, H, H, B, lw, lh, uw, uh, BK, BK * 2));
-                SIS_PROPAGATE(make_im2col_map(&maps.a[i][1], ws.a_lo[call.in_slot], call.cin, H, H, B, lw, lh, uw, uh, BK, BK * 2));
-            }
-        } else {
-            const uint64_t adims[4] = {(uint64_t)call.cin, (uint64_t)H, (uint64_t)H, (uint64_t)B};
-            const uint32_t abox[4] = {(uint32_t)BK, (uint32_t)(halo ? HALO_W : tw), (uint32_t)(halo ? HALO_H : th), (uint32_t)tb};
-            SIS_PROPAGATE(make_map(&maps.a[0][0], ws.a_hi[call.in_slot], 4, adims, abox, BK * 2));
-            SIS_PROPAGATE(make_map(&maps.a[0][1], ws.a_lo[call.in_slot], 4, adims, abox, BK * 2));
-        }
-        const uint64_t wdims[3] = {(uint64_t)call.cin, (uint64_t)call.cout, 9};
-        const uint32_t wbox[3] = {(uint32_t)BK, (uint32_t)(BN / CG), 1};     // CG = 2: each CTA stages half the rows
-        SIS_PROPAGATE(make_map(&maps.w[0], w.hi, 3, wdims, wbox, BK * 2));
-        SIS_PROPAGATE(make_map(&maps.w[1], w.lo, 3, wdims, wbox, BK * 2));
-    }
-    int st;
+    if (halo) SIS_PROPAGATE(make_halo_maps(maps, ws, call, BK, HALO_W, HALO_H));
+    else
+        for (int i = 0; i < a.nsub; ++i) SIS_PROPAGATE(make_im2col_maps(maps, i, a.sub[i], ws, call, BK));
+    SIS_PROPAGATE(make_weight_maps(maps, w.hi, w.lo, call.cin, call.cout, 9, BK, BN / CG));     // CG = 2: each CTA stages half the rows
     {
         ProfScope prof(conv_cat, stream);
-        static int rw_env = env_int("SIS_TC_RW", 1) != 0;
-        if (halo && rw_env && BN == 32 && BK == 32 && CG == 1 && a.kchunks == 1 && n_tiles == 1) st = launch_tc_halo_rw<32, 32, false>(maps, a, stream);
-        else if (halo) st = (CG == 2) ? launch_tc_halo_any<2>(BN, BK, maps, a, stream) : launch_tc_halo_any<1>(BN, BK, maps, a, stream);
-        else if (CG == 2) st = (BK == 64) ? launch_tc_any<64, 2>(BN, th, tw, tb, maps, a, stream) : launch_tc_any<32, 2>(BN, th, tw, tb, maps, a, stream);
-        else st = (BK == 64) ? launch_tc_any<64, 1>(BN, th, tw, tb, maps, a, stream) : launch_tc_any<32, 1>(BN, th, tw, tb, maps, a, stream);
+        if (halo && BN == 32 && BK == 32 && CG == 1 && a.kchunks == 1 && n_tiles == 1)          // 32 -> 32: resident weights
+            SIS_PROPAGATE((launch_persistent<modconv_tc_halo_rw_kernel<32, 32, false>, TcHaloRwCfg<32, 32, false>::SMEM_BYTES>(maps, a, stream)));
+        else if (halo)
+            SIS_PROPAGATE(CG == 2 ? launch_tc_halo<2>(BN, BK, maps, a, stream) : launch_tc_halo<1>(BN, BK, maps, a, stream));
+        else if (CG == 2)
+            SIS_PROPAGATE((BK == 64 ? launch_tc<64, 2>(BN, maps, a, stream) : launch_tc<32, 2>(BN, maps, a, stream)));
+        else
+            SIS_PROPAGATE((BK == 64 ? launch_tc<64, 1>(BN, maps, a, stream) : launch_tc<32, 1>(BN, maps, a, stream)));
     }
-    SIS_PROPAGATE(st);
-
     if (call.up) SIS_PROPAGATE(tc_blur_after_upconv(ws, call, stream));
     return SIS_OK;
 }
@@ -2200,12 +2026,11 @@ int tc_conv1x1(const void* a_hi, const void* a_lo, const void* w_hi, const void*
     TcKernelArgs a;
     memset(&a, 0, sizeof(a));
     a.batch = batch; a.cin = cin; a.cout = cout; a.kchunks = cin / BK;
-    a.b_tiles = batch; a.n_tiles = n_tiles;
-    a.demod = ones; a.error = d_error; a.act = 0; a.im2col = 1; a.mode = out_nhwc ? 1 : 0; a.nsub = 1;
+    a.b_tiles = batch;
+    a.demod = ones; a.error = d_error; a.act = 0; a.mode = out_nhwc ? 1 : 0; a.nsub = 1;
     TcSubProblem& s = a.sub[0];
     s.ntaps = 1; s.dy[0] = 0; s.dx[0] = 0; s.widx[0] = 0;
     s.oh = res; s.ow = res; s.ostride = 1; s.ooff_y = 0; s.ooff_x = 0;
-    s.tiles_y = ceil_div(res, 8); s.tiles_x = ceil_div(res, 16); s.tile_begin = 0;
     s.m_tiles = (int)m_tiles; s.base_dy = 0; s.base_dx = 0;
     a.total_tiles = ceil_div((int)m_tiles, CG) * n_tiles;
     a.out_f32 = out; a.out_h = res; a.out_w = res;
@@ -2213,13 +2038,10 @@ int tc_conv1x1(const void* a_hi, const void* a_lo, const void* w_hi, const void*
     memset(&maps, 0, sizeof(maps));
     SIS_PROPAGATE(make_im2col_map(&maps.a[0][0], const_cast<void*>(a_hi), cin, res, res, batch, 0, 0, 0, 0, BK, BK * 2));
     SIS_PROPAGATE(make_im2col_map(&maps.a[0][1], const_cast<void*>(a_lo), cin, res, res, batch, 0, 0, 0, 0, BK, BK * 2));
-    const uint64_t wdims[3] = {(uint64_t)cin, (uint64_t)cout, 1};
-    const uint32_t wbox[3] = {(uint32_t)BK, (uint32_t)(BN / CG), 1};
-    SIS_PROPAGATE(make_map(&maps.w[0], const_cast<void*>(w_hi), 3, wdims, wbox, BK * 2));
-    SIS_PROPAGATE(make_map(&maps.w[1], const_cast<void*>(w_lo), 3, wdims, wbox, BK * 2));
+    SIS_PROPAGATE(make_weight_maps(maps, w_hi, w_lo, cin, cout, 1, BK, BN / CG));
     ProfScope prof(PROF_CONV_TC, stream);
-    if (CG == 2) return (BK == 64) ? launch_tc_any<64, 2>(BN, 8, 16, 1, maps, a, stream) : launch_tc_any<32, 2>(BN, 8, 16, 1, maps, a, stream);
-    return (BK == 64) ? launch_tc_any<64, 1>(BN, 8, 16, 1, maps, a, stream) : launch_tc_any<32, 1>(BN, 8, 16, 1, maps, a, stream);
+    if (CG == 2) return (BK == 64) ? launch_tc<64, 2>(BN, maps, a, stream) : launch_tc<32, 2>(BN, maps, a, stream);
+    return (BK == 64) ? launch_tc<64, 1>(BN, maps, a, stream) : launch_tc<32, 1>(BN, maps, a, stream);
 }
 
 }  // namespace sis

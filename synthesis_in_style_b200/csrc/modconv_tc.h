@@ -3,7 +3,6 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <map>
-#include <vector>
 
 namespace sis {
 
@@ -14,8 +13,6 @@ struct TcConvWeights {
     int cin = 0, cout = 0;
 };
 
-struct TcTensorMapCacheEntry;   // opaque (CUtensorMap storage)
-
 struct TcWorkspace {
     // A-operand planes: NHWC bf16, pre-multiplied by the consuming conv's style.  Two slots (ping-pong).
     void* a_hi[2] = {nullptr, nullptr};
@@ -23,7 +20,6 @@ struct TcWorkspace {
     size_t a_bytes = 0;
     int batch = -1;
     unsigned int* d_error = nullptr;              // device-side watchdog / error word
-    std::vector<TcTensorMapCacheEntry*> maps;     // cached tensor maps
 };
 
 struct TcConvCall {
