@@ -95,6 +95,13 @@ typedef enum {
 } sis_precision;
 
 SIS_API int sis_generator_create(int size, int style_dim, int n_mlp, int channel_multiplier, sis_generator** out);
+/* SWAGAN generator (scf/networks/swagan/model.py:101-286), size a power of two in [16, 1024]: the StyleGAN2 conv trunk of
+ * size / 2 (log_size = log2(size) - 1, num_layers = 2*log_size - 3, n_latent = 2*log_size - 2, same channel table, noise maps
+ * and activation indices), 12-channel wavelet ToRGBs (keys to_rgb*.conv.weight [1,12,Cin,1,1], to_rgb*.bias [1,12,1,1],
+ * and on the up-sampling ones upsample.kernel, iwt.{ll,lh,hl,hh}, dwt.{ll,lh,hl,hh}) and the generator's own iwt.* for the
+ * final inverse Haar transform.  Every other sis_generator_* function works on the handle unchanged; d_image is
+ * [batch,3,size,size].  Label jobs on an activation that also feeds a ToRGB run as a separate pass. */
+SIS_API int sis_generator_create_swagan(int size, int style_dim, int n_mlp, int channel_multiplier, sis_generator** out);
 SIS_API int sis_generator_destroy(sis_generator* g);
 /* `key` is the reference state-dict key, e.g. "convs.3.conv.modulation.weight". */
 SIS_API int sis_generator_set_param(sis_generator* g, const char* key, const float* d_ptr, int64_t numel);
@@ -159,6 +166,10 @@ SIS_API int sis_generator_check(sis_generator* g, void* stream);
  *                          writes [B,Cout,2res,2res]; noise [1 or B,1,R,R] (stride 0 or R*R) with its scalar weight.
  *   sis_to_rgb             ToRGB.forward (model.py:355-364): 1x1 modulated conv (no demod) + bias [3] + upsampled skip
  *                          [B,3,res/2,res/2] (up_kernel [4,4]) -> [B,3,res,res].
+ *   sis_wavelet_to_rgb     SWAGAN ToRGB.forward (swagan/model.py:84-98), one pass: 1x1 modulated conv (no demod) to 12
+ *                          channels (weight [12,Cin]) + bias [12] + dwt(upsample(iwt(skip))) of the skip [B,12,res/2,res/2]
+ *                          (iwt / dwt taps [4,2,2] in ll, lh, hl, hh order, up_kernel [4,4]) -> [B,12,res,res];
+ *                          res a multiple of 4.
  *   sis_equal_linear       EqualLinear.forward (model.py:152-162), optional fused leaky ReLU.
  *   sis_pixel_norm         PixelNorm.forward (model.py:19-20) over rows of `dim`.
  *   sis_noise_injection    NoiseInjection.forward (model.py:287-292): x + weight * noise.
@@ -171,6 +182,9 @@ SIS_API int sis_modulated_conv2d(const float* d_x, int batch, int cin, int res, 
 SIS_API int sis_to_rgb(const float* d_x, int batch, int cin, int res, const float* d_weight, const float* d_mod_weight,
                        const float* d_mod_bias, int style_dim, const float* d_style, const float* d_bias, const float* d_skip,
                        const float* d_up_kernel, float* d_out, void* stream);
+SIS_API int sis_wavelet_to_rgb(const float* d_x, int batch, int cin, int res, const float* d_weight, const float* d_mod_weight,
+                               const float* d_mod_bias, int style_dim, const float* d_style, const float* d_bias, const float* d_skip,
+                               const float* d_iwt, const float* d_up_kernel, const float* d_dwt, float* d_out, void* stream);
 SIS_API int sis_equal_linear(const float* d_x, int64_t rows, int in_dim, const float* d_weight, const float* d_bias, int out_dim,
                              float lr_mul, int fused_lrelu, float* d_out, void* stream);
 SIS_API int sis_pixel_norm(const float* d_x, float* d_out, int64_t rows, int dim, void* stream);

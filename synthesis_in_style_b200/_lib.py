@@ -60,6 +60,7 @@ _SIGNATURES = {
     'sis_upfirdn2d_out_size': (c_int, [c_int] * 6),
     'sis_upfirdn2d': (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int64] + [c_int] * 13 + [c_void_p]),
     'sis_generator_create': (c_int, [c_int, c_int, c_int, c_int, POINTER(c_void_p)]),
+    'sis_generator_create_swagan': (c_int, [c_int, c_int, c_int, c_int, POINTER(c_void_p)]),
     'sis_generator_destroy': (c_int, [c_void_p]),
     'sis_generator_set_param': (c_int, [c_void_p, c_char_p, c_void_p, c_int64]),
     'sis_generator_prepare': (c_int, [c_void_p, c_void_p]),
@@ -73,6 +74,8 @@ _SIGNATURES = {
                                      c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p]),
     'sis_to_rgb': (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
                            c_void_p, c_void_p]),
+    'sis_wavelet_to_rgb': (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p,
+                                   c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     'sis_equal_linear': (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p, c_int, c_float, c_int, c_void_p, c_void_p]),
     'sis_pixel_norm': (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p]),
     'sis_noise_injection': (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),

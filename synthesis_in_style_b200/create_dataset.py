@@ -86,17 +86,22 @@ def resolve_device(name: str) -> torch.device:
 
 # ---------------------------------------------------------------------------------------------- model / segmenter
 def load_generator(args: argparse.Namespace, config: dict, device) -> Generator:
-    """The decoder of `load_autoencoder_or_generator` (networks/__init__.py:413-423): StyleGAN2 generator of
-    `config['image_size']` / `config['latent_size']`, weights from the checkpoint's 'autoencoder' entry (its `decoder.*`
-    keys) when the config names a `stylegan_checkpoint`, else from 'g_ema'."""
+    """The decoder of `load_autoencoder_or_generator` (networks/__init__.py:413-423): the StyleGAN2 generator
+    (`stylegan_variant` 2, the default) or the SWAGAN generator (`'swagan'`) of `config['image_size']` /
+    `config['latent_size']`, weights from the checkpoint's 'autoencoder' entry (its `decoder.*` keys) when the config
+    names a `stylegan_checkpoint`, else from 'g_ema'."""
     variant = config.get('stylegan_variant', 2)
-    if variant != 2:
-        raise NotImplementedError(f'stylegan_variant {variant!r}: the B200 hot path is the StyleGAN2 generator')
+    if variant == 2:
+        cls = Generator
+    elif variant == 'swagan':
+        from .swagan import Generator as cls
+    else:
+        raise NotImplementedError(f'stylegan_variant {variant!r}: the B200 hot path has the StyleGAN2 and SWAGAN generators')
     ckpt = str(args.checkpoint)
     if ckpt.startswith('random-init:'):
         torch.manual_seed(int(ckpt.split(':', 1)[1]))
-        return Generator(config['image_size'], config['latent_size'], 8, channel_multiplier=2).to(device).eval()
-    generator = Generator(config['image_size'], config['latent_size'], 8, channel_multiplier=2)
+        return cls(config['image_size'], config['latent_size'], 8, channel_multiplier=2).to(device).eval()
+    generator = cls(config['image_size'], config['latent_size'], 8, channel_multiplier=2)
     weights = torch.load(ckpt, map_location='cpu')
     if 'stylegan_checkpoint' in config:
         weights = weights['autoencoder'] if 'autoencoder' in weights else weights

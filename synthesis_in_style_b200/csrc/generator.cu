@@ -1,4 +1,6 @@
-// Host-side plan of the StyleGAN2 generator forward (Generator.forward, scf/networks/stylegan2/model.py:479-561).
+// Host-side plan of the StyleGAN2 generator forward (Generator.forward, scf/networks/stylegan2/model.py:479-561) and of
+// the SWAGAN generator forward (scf/networks/swagan/model.py:200-286: the same conv trunk stopped at size / 2, 12-channel
+// wavelet ToRGBs, and the image as the inverse Haar transform of the last skip).
 // Owns repacked weights and grow-only device workspaces; every forward is a fixed sequence of launches on the
 // caller's stream.  See DESIGN.md for the layer schedule and the data layout in HBM.
 #include <map>
@@ -41,6 +43,7 @@ struct RgbLayer {
     int cin = 0, res = 0; bool up = false;
     std::string prefix;
     DevBuf w_scaled, mod_w, mod_b, bias, up_k;
+    DevBuf iwt_k, dwt_k;     // SWAGAN: [4 bands][2][2] Haar taps of the skip path
     float* s = nullptr;      // [B, cin]
 };
 
@@ -50,6 +53,10 @@ using namespace sis;
 
 struct sis_generator {
     int size = 0, style_dim = 0, n_mlp = 0, channel_multiplier = 2;
+    // variant: StyleGAN2 = 3-channel ToRGBs, trunk at the image size; SWAGAN = 12-channel wavelet ToRGBs, trunk at
+    // size / 2 and the image written by the last ToRGB through the generator's inverse Haar transform (`iwt_k`)
+    int rgb_channels = 3, trunk_size = 0;
+    DevBuf iwt_k;
     int log_size = 0, num_layers = 0, n_latent = 0;
     std::map<int, int> channels;
     std::map<std::string, std::pair<const float*, int64_t>> params;
@@ -75,13 +82,11 @@ static int act_channels(const sis_generator* g, int idx, int* res) {
     return g->channels.at(r);
 }
 
-extern "C" int sis_generator_create(int size, int style_dim, int n_mlp, int channel_multiplier, sis_generator** out) {
-    SIS_REQUIRE(out != nullptr, "generator_create: out is null");
-    SIS_REQUIRE(size >= 8 && size <= 1024 && (size & (size - 1)) == 0, "generator_create: size must be a power of two in [8, 1024] (got %d)", size);
-    SIS_REQUIRE(style_dim >= 1 && n_mlp >= 0 && channel_multiplier >= 1, "generator_create: bad style_dim / n_mlp / channel_multiplier");
+static sis_generator* new_plan(int size, int trunk_size, int rgb_channels, int style_dim, int n_mlp, int channel_multiplier) {
     sis_generator* g = new sis_generator();
     g->size = size; g->style_dim = style_dim; g->n_mlp = n_mlp; g->channel_multiplier = channel_multiplier;
-    g->log_size = (int)std::lround(std::log2((double)size));
+    g->rgb_channels = rgb_channels; g->trunk_size = trunk_size;
+    g->log_size = (int)std::lround(std::log2((double)trunk_size));
     g->num_layers = (g->log_size - 2) * 2 + 1;
     g->n_latent = g->log_size * 2 - 2;
     // Generator.get_channels, model.py:443-455
@@ -105,7 +110,22 @@ extern "C" int sis_generator_create(int size, int style_dim, int n_mlp, int chan
         g->rgbs.push_back(std::move(r));
         cin = cout;
     }
-    *out = g;
+    return g;
+}
+
+extern "C" int sis_generator_create(int size, int style_dim, int n_mlp, int channel_multiplier, sis_generator** out) {
+    SIS_REQUIRE(out != nullptr, "generator_create: out is null");
+    SIS_REQUIRE(size >= 8 && size <= 1024 && (size & (size - 1)) == 0, "generator_create: size must be a power of two in [8, 1024] (got %d)", size);
+    SIS_REQUIRE(style_dim >= 1 && n_mlp >= 0 && channel_multiplier >= 1, "generator_create: bad style_dim / n_mlp / channel_multiplier");
+    *out = new_plan(size, size, 3, style_dim, n_mlp, channel_multiplier);
+    return SIS_OK;
+}
+
+extern "C" int sis_generator_create_swagan(int size, int style_dim, int n_mlp, int channel_multiplier, sis_generator** out) {
+    SIS_REQUIRE(out != nullptr, "generator_create_swagan: out is null");
+    SIS_REQUIRE(size >= 16 && size <= 1024 && (size & (size - 1)) == 0, "generator_create_swagan: size must be a power of two in [16, 1024] (got %d)", size);
+    SIS_REQUIRE(style_dim >= 1 && n_mlp >= 0 && channel_multiplier >= 1, "generator_create_swagan: bad style_dim / n_mlp / channel_multiplier");
+    *out = new_plan(size, size / 2, 12, style_dim, n_mlp, channel_multiplier);
     return SIS_OK;
 }
 
@@ -118,7 +138,10 @@ extern "C" int sis_generator_destroy(sis_generator* g) {
         c.w_scaled.release(); c.wsq.release(); c.mod_w.release(); c.mod_b.release(); c.act_bias.release(); c.blur_k.release();
         tc_free_weights(c.tc);
     }
-    for (auto& r : g->rgbs) { r.w_scaled.release(); r.mod_w.release(); r.mod_b.release(); r.bias.release(); r.up_k.release(); }
+    for (auto& r : g->rgbs) {
+        r.w_scaled.release(); r.mod_w.release(); r.mod_b.release(); r.bias.release(); r.up_k.release(); r.iwt_k.release(); r.dwt_k.release();
+    }
+    g->iwt_k.release();
     DevBuf* bufs[] = {&g->latent, &g->wbuf[0], &g->wbuf[1], &g->mlp_tmp[0], &g->mlp_tmp[1], &g->styles, &g->demods, &g->jobs_dev,
                       &g->act_pp[0], &g->act_pp[1], &g->upconv_tmp, &g->skip_pp[0], &g->skip_pp[1], &g->style_tmp[0],
                       &g->style_tmp[1], &g->style_jobs};
@@ -166,6 +189,18 @@ static int copy_param(sis_generator* g, const std::string& key, int64_t n, DevBu
     return SIS_OK;
 }
 
+// `<prefix>.{ll,lh,hl,hh}` (2x2 each, swagan/model.py:28-68) -> dst [4 bands][2][2]
+static int copy_haar_taps(sis_generator* g, const std::string& prefix, DevBuf& dst, cudaStream_t stream) {
+    SIS_PROPAGATE(dst.reserve(16 * sizeof(float)));
+    const char* bands[4] = {"ll", "lh", "hl", "hh"};
+    for (int i = 0; i < 4; ++i) {
+        const float* src;
+        SIS_PROPAGATE(get_param(g, prefix + "." + bands[i], 4, &src));
+        SIS_CHECK_CUDA(cudaMemcpyAsync(dst.as<float>() + 4 * i, src, 4 * sizeof(float), cudaMemcpyDeviceToDevice, stream));
+    }
+    return SIS_OK;
+}
+
 extern "C" int sis_generator_prepare(sis_generator* g, void* stream_) {
     cudaStream_t stream = (cudaStream_t)stream_;
     SIS_REQUIRE(g != nullptr, "generator_prepare: null generator");
@@ -204,14 +239,20 @@ extern "C" int sis_generator_prepare(sis_generator* g, void* stream_) {
         SIS_CHECK_CUDA(cudaMemcpyAsync(&c.noise_w, nw, sizeof(float), cudaMemcpyDeviceToHost, stream));
         SIS_PROPAGATE(tc_pack_weights(c.tc, w, c.cin, c.cout, c.up, scale, stream));
     }
+    const int rc = g->rgb_channels;
     for (auto& r : g->rgbs) {
         const float scale = (float)(1.0 / std::sqrt((double)r.cin));          // 1x1 kernel: fan_in = cin
-        SIS_PROPAGATE(copy_param(g, r.prefix + ".conv.weight", (int64_t)3 * r.cin, r.w_scaled, scale, stream));
+        SIS_PROPAGATE(copy_param(g, r.prefix + ".conv.weight", (int64_t)rc * r.cin, r.w_scaled, scale, stream));
         SIS_PROPAGATE(copy_param(g, r.prefix + ".conv.modulation.weight", (int64_t)r.cin * sd, r.mod_w, mod_scale, stream));
         SIS_PROPAGATE(copy_param(g, r.prefix + ".conv.modulation.bias", r.cin, r.mod_b, 1.0f, stream));
-        SIS_PROPAGATE(copy_param(g, r.prefix + ".bias", 3, r.bias, 1.0f, stream));
+        SIS_PROPAGATE(copy_param(g, r.prefix + ".bias", rc, r.bias, 1.0f, stream));
         if (r.up) SIS_PROPAGATE(copy_param(g, r.prefix + ".upsample.kernel", 16, r.up_k, 1.0f, stream));
+        if (r.up && rc == 12) {
+            SIS_PROPAGATE(copy_haar_taps(g, r.prefix + ".iwt", r.iwt_k, stream));
+            SIS_PROPAGATE(copy_haar_taps(g, r.prefix + ".dwt", r.dwt_k, stream));
+        }
     }
+    if (rc == 12) SIS_PROPAGATE(copy_haar_taps(g, "iwt", g->iwt_k, stream));
     SIS_CHECK_CUDA(cudaStreamSynchronize(stream));  // noise weights and blur taps are read on the host
     for (auto& c : g->convs) {
         if (!c.up) continue;
@@ -405,7 +446,7 @@ extern "C" int sis_generator_forward(sis_generator* g, const sis_forward_args* a
         if (a->d_activations && a->d_activations[idx]) return a->d_activations[idx];
         return g->act_pp[pp].as<float>();
     };
-    if (tc) SIS_PROPAGATE(tc_ensure_workspace(g->tc_ws, B, g->size, g->channels[4], g->channels));
+    if (tc) SIS_PROPAGATE(tc_ensure_workspace(g->tc_ws, B, g->trunk_size, g->channels[4], g->channels));
 
     float* x = act_dst(0, 0);
     SIS_PROPAGATE(launch_const_input(x, g->const_input.as<float>(), (int64_t)g->channels[4] * 16, B, stream));
@@ -452,7 +493,23 @@ extern "C" int sis_generator_forward(sis_generator* g, const sis_forward_args* a
             }
         }
         x = y; pp ^= 1;
-        if (L % 2 == 0) {  // ToRGB after conv1 and after the second conv of every block (model.py:538,550)
+        if (L % 2 == 0 && g->rgb_channels == 12) {   // SWAGAN ToRGB (swagan/model.py:253-284); labelling runs unfused
+            RgbLayer& r = g->rgbs[rgb_i];
+            const bool last = rgb_i + 1 == (int)g->rgbs.size();
+            SIS_PROPAGATE(run_label_jobs(a, (int)L + 1, x, B, c.cout, c.res_out, nullptr, nullptr, stream));
+            WaveletToRgbArgs t;
+            t.x = x; t.s = r.s; t.w = r.w_scaled.as<float>(); t.bias = r.bias.as<float>(); t.skip = skip;
+            t.iwt_k = r.iwt_k.as<float>(); t.up_k = r.up_k.as<float>(); t.dwt_k = r.dwt_k.as<float>();
+            t.final_iwt_k = last ? g->iwt_k.as<float>() : nullptr;     // the last one writes the image (:285)
+            t.out = last ? a->d_image : g->skip_pp[rgb_i & 1].as<float>();
+            t.batch = B; t.C = r.cin; t.H = r.res; t.W = r.res;
+            {
+                ProfScope prof(PROF_TORGB, stream);
+                SIS_PROPAGATE(launch_wavelet_torgb(t, stream));
+            }
+            skip = t.out;
+            ++rgb_i;
+        } else if (L % 2 == 0) {  // ToRGB after conv1 and after the second conv of every block (model.py:538,550)
             RgbLayer& r = g->rgbs[rgb_i];
             const bool last = rgb_i + 1 == (int)g->rgbs.size();
             float* out = last ? a->d_image : g->skip_pp[rgb_i & 1].as<float>();

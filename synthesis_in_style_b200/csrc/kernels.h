@@ -44,6 +44,21 @@ struct ToRgbArgs {
     int batch, C, H, W;
 };
 
+// SWAGAN ToRGB (wavelet_torgb.cu): 12 output channels = 4 Haar bands x RGB
+struct WaveletToRgbArgs {
+    const float* x;            // [B, C, H, W]
+    const float* s;            // [B, C]
+    const float* w;            // [12, C] pre-scaled
+    const float* bias;         // [12]
+    const float* skip;         // [B, 12, H/2, W/2] or null
+    const float* iwt_k;        // [4 bands][2][2] inverse Haar taps applied to the skip
+    const float* up_k;         // [4][4]
+    const float* dwt_k;        // [4 bands][2][2]
+    const float* final_iwt_k;  // [4 bands][2][2] or null: write the image [B, 3, 2H, 2W] instead of [B, 12, H, W]
+    float* out;
+    int batch, C, H, W;
+};
+
 struct LabelArgs {
     const float* act; int batch, C, H, W;
     const float* centroids; int k;
@@ -69,5 +84,6 @@ int launch_modconv3x3_simt(const ModConvSimtArgs& a, int batch, cudaStream_t str
 int launch_const_input(float* out, const float* inp, int64_t per_sample, int batch, cudaStream_t stream);
 int launch_blur_noise_act(const BlurActArgs& a, cudaStream_t stream);
 int launch_torgb(const ToRgbArgs& a, cudaStream_t stream);
+int launch_wavelet_torgb(const WaveletToRgbArgs& a, cudaStream_t stream);
 
 }  // namespace sis

@@ -126,6 +126,30 @@ extern "C" int sis_to_rgb(const float* d_x, int batch, int cin, int res, const f
     return launch_torgb(t, stream);
 }
 
+extern "C" int sis_wavelet_to_rgb(const float* d_x, int batch, int cin, int res, const float* d_weight, const float* d_mod_weight,
+                                  const float* d_mod_bias, int style_dim, const float* d_style, const float* d_bias, const float* d_skip,
+                                  const float* d_iwt, const float* d_up_kernel, const float* d_dwt, float* d_out, void* stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    SIS_REQUIRE(batch >= 0 && cin >= 1 && res >= 1 && style_dim >= 1, "wavelet_to_rgb: bad shape");
+    if (batch == 0) return SIS_OK;
+    SIS_REQUIRE(d_x && d_weight && d_mod_weight && d_mod_bias && d_style && d_bias && d_out, "wavelet_to_rgb: input must be a CUDA tensor (null pointer)");
+    SIS_REQUIRE(!d_skip || (d_iwt && d_up_kernel && d_dwt), "wavelet_to_rgb: a skip needs the iwt, upsample and dwt taps");
+    SIS_REQUIRE(res % 4 == 0, "wavelet_to_rgb: resolution must be a multiple of 4 (got %d)", res);
+    LayerScratch& L = g_ls;
+    SIS_PROPAGATE(L.mod_w.reserve((size_t)cin * style_dim * sizeof(float)));
+    SIS_PROPAGATE(launch_scale_copy(L.mod_w.as<float>(), d_mod_weight, (float)(1.0 / std::sqrt((double)style_dim)), (int64_t)cin * style_dim, stream));
+    SIS_PROPAGATE(L.s.reserve((size_t)batch * cin * sizeof(float)));
+    SIS_PROPAGATE(run_linear(d_style, style_dim, L.mod_w.as<float>(), d_mod_bias, L.s.as<float>(), cin, batch, cin, style_dim, 0, LINEAR_EPI_BIAS, stream));
+    SIS_PROPAGATE(L.w_scaled.reserve((size_t)12 * cin * sizeof(float)));
+    SIS_PROPAGATE(launch_scale_copy(L.w_scaled.as<float>(), d_weight, (float)(1.0 / std::sqrt((double)cin)), (int64_t)12 * cin, stream));
+    WaveletToRgbArgs t;
+    t.x = d_x; t.s = L.s.as<float>(); t.w = L.w_scaled.as<float>(); t.bias = d_bias; t.skip = d_skip;
+    t.iwt_k = d_iwt; t.up_k = d_up_kernel; t.dwt_k = d_dwt; t.final_iwt_k = nullptr;
+    t.out = d_out; t.batch = batch; t.C = cin; t.H = res; t.W = res;
+    ProfScope prof(PROF_TORGB, stream);
+    return launch_wavelet_torgb(t, stream);
+}
+
 extern "C" int sis_modulated_conv2d(const float* d_x, int batch, int cin, int res, const float* d_weight, int cout,
                                     const float* d_mod_weight, const float* d_mod_bias, int style_dim, const float* d_style,
                                     int demodulate, int upsample, const float* d_blur_kernel, const float* d_noise,

@@ -268,44 +268,20 @@ class _StyleMLP(nn.Module):
         return self._owner[0]._style(z)
 
 
-class Generator(nn.Module):
-    def __init__(self, size, style_dim, n_mlp, channel_multiplier=2, blur_kernel=(1, 3, 3, 1), lr_mlp=0.01,
-                 precision='bf16x3'):
-        super().__init__()
+class _PlanGenerator(nn.Module):
+    """The native plan behind a generator with the reference's call surface: the StyleGAN2 `Generator` below and
+    `swagan.Generator`.  A subclass builds the reference's module tree (the state dict the plan reads) with the attributes
+    `size, style_dim, n_mlp, channel_multiplier, channels, log_size, num_layers, n_latent, precision, input`, a `_StyleMLP`
+    as `style` and `_plan = _Plan()`, and names the C-ABI call that creates its plan in `_CREATE`."""
+
+    _CREATE = 'sis_generator_create'
+
+    @staticmethod
+    def _require_plan_defaults(blur_kernel, lr_mlp):
         if list(blur_kernel) != [1, 3, 3, 1]:
             raise NotImplementedError('the fused plan is built for the reference default blur_kernel=[1, 3, 3, 1]')
         if lr_mlp != 0.01:
             raise NotImplementedError('the fused plan is built for the reference default lr_mlp=0.01')
-        self.size, self.style_dim = size, style_dim
-        self.n_mlp, self.channel_multiplier = n_mlp, channel_multiplier
-        self.precision = precision
-        self.style = _StyleMLP(style_dim, n_mlp, lr_mlp)
-        self.style._owner = (self,)   # tuple: not registered as a sub-module
-        self.channels = self.get_channels(channel_multiplier)
-        self.input = ConstantInput(self.channels[4])
-        self.conv1 = StyledConv(self.channels[4], self.channels[4], 3, style_dim, blur_kernel=blur_kernel)
-        self.to_rgb1 = ToRGB(self.channels[4], style_dim, upsample=False)
-        self.log_size = int(math.log(size, 2))
-        self.num_layers = (self.log_size - 2) * 2 + 1
-        self.convs = nn.ModuleList()
-        self.upsamples = nn.ModuleList()
-        self.to_rgbs = nn.ModuleList()
-        self.noises = nn.Module()
-        in_channel = self.channels[4]
-        for layer_idx in range(self.num_layers):
-            res = (layer_idx + 5) // 2
-            self.noises.register_buffer(f'noise_{layer_idx}', torch.randn(1, 1, 2 ** res, 2 ** res))
-        for i in range(3, self.log_size + 1):
-            out_channel = self.channels[2 ** i]
-            self.convs.append(StyledConv(in_channel, out_channel, 3, style_dim, upsample=True, blur_kernel=blur_kernel))
-            self.convs.append(StyledConv(out_channel, out_channel, 3, style_dim, blur_kernel=blur_kernel))
-            self.to_rgbs.append(ToRGB(out_channel, style_dim))
-            in_channel = out_channel
-        self.n_latent = self.log_size * 2 - 2
-        for m in self.modules():
-            if isinstance(m, ModulatedConv2d):
-                m.precision = precision      # stand-alone layer calls follow the generator's precision
-        self._plan = _Plan()
 
     # ------------------------------------------------------------------ reference helpers
     @staticmethod
@@ -364,8 +340,8 @@ class Generator(nn.Module):
         with torch.cuda.device(dev):
             if self._plan.handle is None:
                 h = ctypes.c_void_p()
-                _lib.check(lib.sis_generator_create(self.size, self.style_dim, self.n_mlp, self.channel_multiplier,
-                                                    ctypes.byref(h)))
+                _lib.check(getattr(lib, self._CREATE)(self.size, self.style_dim, self.n_mlp, self.channel_multiplier,
+                                                      ctypes.byref(h)))
                 self._plan.handle = h
             keep = []
             for name, t in state:
@@ -402,7 +378,7 @@ class Generator(nn.Module):
         """Same arguments / returns as the reference (model.py:479-561).  Two optional extensions (not in the reference):
         `capture_layers` restricts which activation indices are materialised when `return_intermediate_activations`;
         `label_jobs` (a list of `labelling.LabelJobSpec`) labels activations inside the same native call, fused with
-        the ToRGB pass where both read the same tensor."""
+        the StyleGAN2 ToRGB pass where both read the same tensor."""
         if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
             # The fused plan is inference-only.  Running silently without a graph would be a wrong gradient.
             raise RuntimeError('Generator.forward of synthesis_in_style_b200 is inference-only: call it under '
@@ -514,3 +490,40 @@ class Generator(nn.Module):
         if return_intermediate_activations:
             return image, acts
         return image, None
+
+
+class Generator(_PlanGenerator):
+    def __init__(self, size, style_dim, n_mlp, channel_multiplier=2, blur_kernel=(1, 3, 3, 1), lr_mlp=0.01,
+                 precision='bf16x3'):
+        super().__init__()
+        self._require_plan_defaults(blur_kernel, lr_mlp)
+        self.size, self.style_dim = size, style_dim
+        self.n_mlp, self.channel_multiplier = n_mlp, channel_multiplier
+        self.precision = precision
+        self.style = _StyleMLP(style_dim, n_mlp, lr_mlp)
+        self.style._owner = (self,)   # tuple: not registered as a sub-module
+        self.channels = self.get_channels(channel_multiplier)
+        self.input = ConstantInput(self.channels[4])
+        self.conv1 = StyledConv(self.channels[4], self.channels[4], 3, style_dim, blur_kernel=blur_kernel)
+        self.to_rgb1 = ToRGB(self.channels[4], style_dim, upsample=False)
+        self.log_size = int(math.log(size, 2))
+        self.num_layers = (self.log_size - 2) * 2 + 1
+        self.convs = nn.ModuleList()
+        self.upsamples = nn.ModuleList()
+        self.to_rgbs = nn.ModuleList()
+        self.noises = nn.Module()
+        in_channel = self.channels[4]
+        for layer_idx in range(self.num_layers):
+            res = (layer_idx + 5) // 2
+            self.noises.register_buffer(f'noise_{layer_idx}', torch.randn(1, 1, 2 ** res, 2 ** res))
+        for i in range(3, self.log_size + 1):
+            out_channel = self.channels[2 ** i]
+            self.convs.append(StyledConv(in_channel, out_channel, 3, style_dim, upsample=True, blur_kernel=blur_kernel))
+            self.convs.append(StyledConv(out_channel, out_channel, 3, style_dim, blur_kernel=blur_kernel))
+            self.to_rgbs.append(ToRGB(out_channel, style_dim))
+            in_channel = out_channel
+        self.n_latent = self.log_size * 2 - 2
+        for m in self.modules():
+            if isinstance(m, ModulatedConv2d):
+                m.precision = precision      # stand-alone layer calls follow the generator's precision
+        self._plan = _Plan()

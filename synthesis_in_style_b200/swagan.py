@@ -1,23 +1,22 @@
-"""SWAGAN generator with the reference's call surface (SURVEY.md §8(f) row 4), composed from the B200 layer entry points.
+"""SWAGAN generator with the reference's call surface (SURVEY.md §8(f) row 4), executed by the fused sm_100a plan.
 
 Mirrors scf/networks/swagan/model.py:14-286: `HaarTransform`, `InverseHaarTransform`, the 12-channel wavelet `ToRGB` and
 `Generator` (constructor signature, attributes, state-dict keys, random-init draw order, `forward` keywords and return
 convention; the conv trunk stops at size / 2 and the image is the inverse Haar transform of the last skip).
-The reference builds it from the StyleGAN2 modules (swagan/model.py:12); so does this file: every StyledConv is one
-`sis_modulated_conv2d` call (tcgen05 GEMM with the fused epilogue), the style MLP is `sis_pixel_norm` + `sis_equal_linear`,
-the wavelet filters are the drop-in `upfirdn2d` op (bit-exact against the reference's kernel on the 2x2 Haar modes,
-tests/test_ref_kernels_gpu.py), and the 12-channel ToRGB is four `sis_to_rgb` calls over its weight slices.
-Layer-per-call, not the fused plan of `model.Generator`: this row is built for parity first (tests/test_swagan_gpu.py).
-Inference only; no CPU path.
+`Generator.forward` is one `sis_generator_forward` call on a plan made by `sis_generator_create_swagan`: the conv trunk,
+style MLP and labelling kernels of the StyleGAN2 plan (the trunk of SWAGAN-S is the trunk of StyleGAN2-S/2), and one
+wavelet ToRGB launch per resolution, the last of which writes the image.  Everything else (activation capture, in-forward
+labelling, `check`, `precision`, copies) is `model.Generator`'s.  Stand-alone, `ToRGB` is one `sis_wavelet_to_rgb` call
+and the Haar modules are the drop-in `upfirdn2d` op.  Inference only; no CPU path.  GPU tests: tests/test_swagan.py,
+tests/test_swagan_plan.py.
 """
 import math
-import random
 
 import torch
 from torch import nn
 
 from . import _lib
-from .model import ConstantInput, EqualLinear, ModulatedConv2d, PixelNorm, StyledConv, _FirBuffer, _f32c, _stream
+from .model import ConstantInput, ModulatedConv2d, StyledConv, _FirBuffer, _f32c, _Plan, _PlanGenerator, _StyleMLP, _stream
 from .op import upfirdn2d
 
 
@@ -72,36 +71,41 @@ class ToRGB(nn.Module):
         self.bias = nn.Parameter(torch.zeros(1, 3 * 4, 1, 1))
 
     def forward(self, input, style, skip=None):
+        """swagan/model.py:84-98 through `sis_wavelet_to_rgb`: 1x1 modulated conv, bias and the skip chain in one pass."""
         x, st = _f32c(input, 'input'), _f32c(style, 'style')
         b, cin, h, _ = x.shape
-        weight = _f32c(self.conv.weight.detach(), 'weight').reshape(12, cin)
-        bias = _f32c(self.bias.detach(), 'bias').reshape(12)
+        sk = _f32c(skip, 'skip') if skip is not None else None
+        if sk is not None and (not hasattr(self, 'upsample') or tuple(sk.shape) != (b, 12, h // 2, h // 2)):
+            raise RuntimeError('skip must be [B, 12, H/2, H/2] and the layer must have been built with upsample=True')
+        taps = {}
+        if hasattr(self, 'upsample'):
+            for name in ('iwt', 'dwt'):
+                m = getattr(self, name)
+                taps[name] = _f32c(torch.stack([m.ll, m.lh, m.hl, m.hh]), f'{name} taps')
+            taps['up'] = _f32c(self.upsample.kernel, 'upsample.kernel')
         mw, mb = _f32c(self.conv.modulation.weight.detach(), 'weight'), _f32c(self.conv.modulation.bias.detach(), 'bias')
-        bands = []
-        lib = _lib.load()
+        out = torch.empty(b, 12, h, h, device=x.device)
         with torch.cuda.device(x.device):
-            for j in range(4):          # one wavelet band (3 channels) per call of the 3-channel ToRGB kernel
-                out = torch.empty(b, 3, h, h, device=x.device)
-                _lib.check(lib.sis_to_rgb(_lib.ptr(x), b, cin, h, _lib.ptr(weight[3 * j:3 * j + 3].contiguous()), _lib.ptr(mw), _lib.ptr(mb),
-                                          mw.shape[1], _lib.ptr(st), _lib.ptr(bias[3 * j:3 * j + 3].contiguous()), None, None,
-                                          _lib.ptr(out), _stream(x)))
-                bands.append(out)
-        out = torch.cat(bands, 1)
-        if skip is not None:
-            out = out + self.dwt(self.upsample(self.iwt(skip)))
+            _lib.check(_lib.load().sis_wavelet_to_rgb(
+                _lib.ptr(x), b, cin, h, _lib.ptr(_f32c(self.conv.weight.detach(), 'weight')), _lib.ptr(mw), _lib.ptr(mb), mw.shape[1],
+                _lib.ptr(st), _lib.ptr(_f32c(self.bias.detach(), 'bias')), _lib.ptr(sk), _lib.ptr(taps.get('iwt')),
+                _lib.ptr(taps.get('up')), _lib.ptr(taps.get('dwt')), _lib.ptr(out), _stream(x)))
         return out
 
 
-class Generator(nn.Module):
+class Generator(_PlanGenerator):
+    """swagan/model.py:101-286 on the plan of `sis_generator_create_swagan` (see `model.Generator` for the forward)."""
+
+    _CREATE = 'sis_generator_create_swagan'
+
     def __init__(self, size, style_dim, n_mlp, channel_multiplier=2, blur_kernel=(1, 3, 3, 1), lr_mlp=0.01, precision='bf16x3'):
         super().__init__()
+        self._require_plan_defaults(blur_kernel, lr_mlp)
         self.size, self.style_dim = size, style_dim
-        layers = [PixelNorm()]
-        for _ in range(n_mlp):
-            layers.append(EqualLinear(style_dim, style_dim, lr_mul=lr_mlp, activation='fused_lrelu'))
-        self.style = nn.Sequential(*layers)
-        self.channels = {4: 512, 8: 512, 16: 512, 32: 512, 64: 256 * channel_multiplier, 128: 128 * channel_multiplier,
-                         256: 64 * channel_multiplier, 512: 32 * channel_multiplier, 1024: 16 * channel_multiplier}
+        self.n_mlp, self.channel_multiplier = n_mlp, channel_multiplier
+        self.style = _StyleMLP(style_dim, n_mlp, lr_mlp)
+        self.style._owner = (self,)   # tuple: not registered as a sub-module
+        self.channels = self.get_channels(channel_multiplier)
         self.input = ConstantInput(self.channels[4])
         self.conv1 = StyledConv(self.channels[4], self.channels[4], 3, style_dim, blur_kernel=blur_kernel)
         self.to_rgb1 = ToRGB(self.channels[4], style_dim, upsample=False)
@@ -126,64 +130,5 @@ class Generator(nn.Module):
         self.precision = precision
         for m in self.modules():
             if isinstance(m, ModulatedConv2d):
-                m.precision = precision
-
-    def make_noise(self):
-        device = self.input.input.device
-        noises = [torch.randn(1, 1, 2 ** 2, 2 ** 2, device=device)]
-        for i in range(3, self.log_size + 1):
-            for _ in range(2):
-                noises.append(torch.randn(1, 1, 2 ** i, 2 ** i, device=device))
-        return noises
-
-    def mean_latent(self, n_latent):
-        latent_in = torch.randn(n_latent, self.style_dim, device=self.input.input.device)
-        return self.style(latent_in).mean(0, keepdim=True)
-
-    def get_latent(self, input):
-        return self.style(input)
-
-    def forward(self, styles, return_latents=False, inject_index=None, truncation=1, truncation_latent=None, input_is_latent=False,
-                noise=None, randomize_noise=True, return_intermediate_activations=False):
-        if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
-            raise RuntimeError('Generator.forward of synthesis_in_style_b200 is inference-only: call it under torch.no_grad()')
-        for s in styles:
-            _lib.require_cuda(s, 'styles')
-        if not input_is_latent:
-            styles = [self.style(s) for s in styles]
-        if noise is None:
-            noise = [None] * self.num_layers if randomize_noise else [getattr(self.noises, f'noise_{i}') for i in range(self.num_layers)]
-        if truncation < 1:
-            styles = [truncation_latent + truncation * (s - truncation_latent) for s in styles]
-        if len(styles) < 2:
-            inject_index = self.n_latent
-            latent = styles[0].unsqueeze(1).repeat(1, inject_index, 1) if styles[0].ndim < 3 else styles[0]
-        else:
-            if inject_index is None:
-                inject_index = random.randint(1, self.n_latent - 1)
-            latent = torch.cat([styles[0].unsqueeze(1).repeat(1, inject_index, 1),
-                                styles[1].unsqueeze(1).repeat(1, self.n_latent - inject_index, 1)], 1)
-        acts = {} if return_intermediate_activations else None
-        out = self.input(latent)
-        if acts is not None:
-            acts[0] = out.detach().clone()
-        out = self.conv1(out, latent[:, 0], noise=noise[0])
-        if acts is not None:
-            acts[1] = out
-        skip = self.to_rgb1(out, latent[:, 1])
-        i = 1
-        for conv1, conv2, noise1, noise2, to_rgb in zip(self.convs[::2], self.convs[1::2], noise[1::2], noise[2::2], self.to_rgbs):
-            out = conv1(out, latent[:, i], noise=noise1)
-            if acts is not None:
-                acts[i + 1] = out
-            out = conv2(out, latent[:, i + 1], noise=noise2)
-            if acts is not None:
-                acts[i + 2] = out
-            skip = to_rgb(out, latent[:, i + 2], skip)
-            i += 2
-        image = self.iwt(skip)
-        if return_latents:
-            return image, latent
-        if return_intermediate_activations:
-            return image, acts
-        return image, None
+                m.precision = precision      # stand-alone layer calls follow the generator's precision
+        self._plan = _Plan()
