@@ -9,6 +9,7 @@ b mod world_size, every rank replays the single reference RNG stream (CPU latent
 its own batches, so the union over ranks equals the reference's single-process run on the same seed.  The only
 collective is one all-reduce of an int64 statistics vector (NCCL on GPUs, gloo in the CPU tests).
 """
+import contextlib
 from dataclasses import dataclass
 from typing import Dict, Iterable, Iterator, List, Optional, Tuple
 
@@ -143,7 +144,6 @@ class LabelledBatch:
     masks: Dict[str, Dict[str, torch.Tensor]]  # PredictedClusters at S x S (bool)
     activations: Dict[int, torch.Tensor]
     ids: Optional[Dict[str, torch.Tensor]] = None      # {layer: uint8 [B, H, H]} cluster ids at native resolution
-    margins: Optional[Dict[str, torch.Tensor]] = None  # {layer: fp32 [B, H, H]} d2 - d1 (only with want_margin)
 
 
 @dataclass
@@ -169,13 +169,25 @@ class SegmentedBatch:
         return numpy.delete(self.images, self.image_ids_to_drop, axis=0), numpy.delete(self.label_images, self.image_ids_to_drop, axis=0)
 
 
+@dataclass
+class _Step:
+    """The device results of one generate -> label step (`LabelledPairGenerator._step`)."""
+    batch_index: int
+    latents: Latents                         # on the device
+    activations: Dict[int, torch.Tensor]
+    image: torch.Tensor                      # [B, 3, S, S] fp32, or uint8 [B, S, S, 3] (image_u8=True)
+    stacked: Dict[str, Tuple[List[str], torch.Tensor]]  # {layer: (class names, uint8 [n_class, B, S, S])}, merged keys included
+    ids: Dict[str, torch.Tensor]             # {layer: uint8 [B, H, H]}
+    lane: int
+    event: torch.cuda.Event                  # recorded on the lane's stream behind the step's last kernel
+
+
 class LabelledPairGenerator:
     """GPU part of `build_dataset`'s loop: generate -> label, per batch, for this rank's shard."""
 
     def __init__(self, generator: Generator, segmenter: ClusterSegmenter, config: Dict, seed: int = 1,
                  mean_latent: Optional[torch.Tensor] = None, rank: int = 0, world_size: int = 1,
-                 capture_only_labelled: bool = False, fused_labelling: bool = True, in_flight: int = 1,
-                 want_margin: bool = False, mix_inject_index: Optional[int] = None):
+                 capture_only_labelled: bool = False, in_flight: int = 1, mix_inject_index: Optional[int] = None):
         """`in_flight` > 1 keeps that many batches in flight on as many CUDA streams, each with its own generator
         workspace (a replica of `generator`: same weights, separate native plan).  Batches are independent, so the
         latency-bound head of one step (mapping network, 4^2..16^2 layers) overlaps the tensor-bound body of the other;
@@ -183,8 +195,6 @@ class LabelledPairGenerator:
         self.generator, self.segmenter = generator, segmenter
         self.in_flight = max(1, int(in_flight))
         self._replicas, self._streams = None, None
-        self.fused_labelling = fused_labelling
-        self.want_margin = want_margin      # fused jobs also write the nearest-centroid margin (parity checks)
         self.mix_inject_index = mix_inject_index
         self.replay_stream = False          # True: every rank replays every draw instead of addressing the streams by position
         self.config, self.seed, self.mean_latent = config, seed, mean_latent
@@ -219,45 +229,48 @@ class LabelledPairGenerator:
             if t is not None and t.is_cuda:
                 t.record_stream(current)
 
+    def _step(self, lanes, lane: int, latent_stream, z: Optional[torch.Tensor] = None, image_u8: bool = False) -> _Step:
+        """Generate and label this rank's next batch on lane `lane`.  Everything is enqueued on the lane's stream: the
+        noise draw (in the reference's order), the generator pass with its in-forward label jobs and the merge of the
+        `keys_to_merge` layers; `event` marks its end.  `z` (pinned [B, latent_size]) stages the latents for an
+        asynchronous copy in; it must not be rewritten before that copy has run."""
+        device = self.generator.input.input.device
+        seg = self.segmenter
+        g, st = lanes[lane]
+        with (torch.cuda.stream(st) if st is not None else contextlib.nullcontext()):
+            idx, latents = next(latent_stream)
+            if z is not None:
+                z.copy_(latents.latent)
+                latents = Latents(z.to(device, non_blocking=True), latents.noise)
+            # labelling runs inside the generator's native call (one pass over each labelled activation)
+            jobs = seg.make_label_jobs(g, latents.latent.shape[0])
+            acts, image = generate_images(latents, g, device=device, mean_latent=self.mean_latent, capture_layers=self.capture_layers,
+                                          label_jobs=jobs, mix_inject_index=self.mix_inject_index)
+            stacked = seg.merge_stacked(seg.jobs_to_stacked(jobs))   # merged destination keys (black_white...segmenter.py:31-40)
+            if image_u8:
+                image = make_image(image)              # uint8 NHWC on the device: a quarter of the fp32 copy
+            event = torch.cuda.Event()
+            event.record(torch.cuda.current_stream(device))
+        self.stats['pairs'] += image.shape[0]
+        self.stats['batches'] += 1
+        return _Step(idx, latents, acts, image, stacked, seg.jobs_to_ids(jobs), lane, event)
+
     def __iter__(self) -> Iterator[LabelledBatch]:
         import collections
-        import contextlib
         device = self.generator.input.input.device
         lanes = self._lanes(device)
         pending = collections.deque()
         stream = sharded_latent_stream(self.generator, self.config, self.seed, self.rank, self.world_size, self.replay_stream)
         n = 0
         while True:
-            g, st = lanes[n % len(lanes)]
-            with (torch.cuda.stream(st) if st is not None else contextlib.nullcontext()):
-                idx, latents = next(stream)          # the noise is drawn on this lane's stream, in the reference's order
-                if self.fused_labelling:
-                    # labelling runs inside the generator's native call (one pass over each labelled activation)
-                    jobs = self.segmenter.make_label_jobs(g, latents.latent.shape[0], want_margin=self.want_margin)
-                    acts, image = generate_images(latents, g, device=device, mean_latent=self.mean_latent,
-                                                  capture_layers=self.capture_layers, label_jobs=jobs,
-                                                  mix_inject_index=self.mix_inject_index)
-                    masks = self.segmenter._as_predicted(self.segmenter.jobs_to_stacked(jobs))
-                    ids, margins = self.segmenter.jobs_to_ids(jobs), self.segmenter.jobs_to_margins(jobs)
-                else:
-                    acts, image = generate_images(latents, g, device=device, mean_latent=self.mean_latent,
-                                                  capture_layers=self.capture_layers, mix_inject_index=self.mix_inject_index)
-                    ids, margins = {}, None
-                    masks = self.segmenter._as_predicted(self.segmenter.label_layers_stacked(acts, ids_out=ids))
-                masks = self.segmenter.merge_sub_images(masks)
-                done = None
-                if st is not None:
-                    done = torch.cuda.Event()
-                    done.record(st)
-            self.stats['pairs'] += image.shape[0]
-            self.stats['batches'] += 1
-            pending.append((LabelledBatch(idx, image, masks, acts, ids, margins), done))
+            s = self._step(lanes, n % len(lanes), stream)
+            pending.append((LabelledBatch(s.batch_index, s.image, self.segmenter._as_predicted(s.stacked), s.activations, s.ids),
+                            s.event))
             n += 1
             if len(pending) >= len(lanes):
                 batch, done = pending.popleft()
-                if done is not None:
+                if len(lanes) > 1:                   # the lanes run on streams of their own
                     self._hand_over([batch.image] + list(batch.activations.values()) + list(batch.ids.values())
-                                    + list((batch.margins or {}).values())
                                     + [m for per_class in batch.masks.values() for m in per_class.values()], done, device)
                 yield batch
 
@@ -266,12 +279,10 @@ class LabelledPairGenerator:
         latents are staged in pinned memory and copied in, the fp32 image and the per-layer uint8 mask stacks are
         copied out to pinned memory on a side stream, with `depth` batches in flight so the copies overlap the next
         batch's kernels.  A yielded HostBatch stays valid until the next one is requested."""
-        import contextlib
         device = self.generator.input.input.device
-        g, seg = self.generator, self.segmenter
         lanes = self._lanes(device)
         depth = max(depth, len(lanes))
-        B, S = self.config['batch_size'], g.size
+        B, S = self.config['batch_size'], self.generator.size
         copy_stream = torch.cuda.Stream(device=device)
         slots = [{'z': torch.empty(B, self.config['latent_size']).pin_memory(),
                   'image': (torch.empty(B, S, S, 3, dtype=torch.uint8) if image_u8 else torch.empty(B, 3, S, S)).pin_memory(),
@@ -284,49 +295,27 @@ class LabelledPairGenerator:
             return HostBatch(slot['index'], slot['image'], dict(slot['masks']), slot['names'], dict(slot['ids']))
 
         n = 0
-        latent_stream = sharded_latent_stream(g, self.config, self.seed, self.rank, self.world_size, self.replay_stream)
+        latent_stream = sharded_latent_stream(self.generator, self.config, self.seed, self.rank, self.world_size, self.replay_stream)
         while True:
             slot = slots[n % (depth + 1)]
-            g, st = lanes[n % len(lanes)]
-            with (torch.cuda.stream(st) if st is not None else contextlib.nullcontext()):
-                idx, latents = next(latent_stream)
-                slot['z'].copy_(latents.latent)
-                lat = Latents(slot['z'].to(device, non_blocking=True), latents.noise)
-                if self.fused_labelling:
-                    jobs = seg.make_label_jobs(g, B)
-                    acts, image = generate_images(lat, g, device=device, mean_latent=self.mean_latent, capture_layers=self.capture_layers,
-                                                  label_jobs=jobs, mix_inject_index=self.mix_inject_index)
-                    stacked, ids = seg.jobs_to_stacked(jobs), seg.jobs_to_ids(jobs)
-                else:
-                    acts, image = generate_images(lat, g, device=device, mean_latent=self.mean_latent, capture_layers=self.capture_layers,
-                                                  mix_inject_index=self.mix_inject_index)
-                    ids = {}
-                    stacked = seg.label_layers_stacked(acts, ids_out=ids)
-                if seg.keys_to_merge:
-                    stacked = seg.merge_stacked(stacked)   # merged destination keys (black_white...segmenter.py:31-40)
-                if image_u8:
-                    image = make_image(image)              # uint8 NHWC on the device: a quarter of the fp32 copy
-                ready = torch.cuda.Event()
-                ready.record(torch.cuda.current_stream(device))
+            s = self._step(lanes, n % len(lanes), latent_stream, slot['z'], image_u8)
             with torch.cuda.stream(copy_stream):
-                copy_stream.wait_event(ready)
-                slot['image'].copy_(image, non_blocking=True)
-                for layer, (names, m) in stacked.items():
+                copy_stream.wait_event(s.event)
+                slot['image'].copy_(s.image, non_blocking=True)
+                for layer, (names, m) in s.stacked.items():
                     if layer not in slot['masks']:
                         slot['masks'][layer] = torch.empty(m.shape, dtype=torch.uint8).pin_memory()
                     slot['masks'][layer].copy_(m, non_blocking=True)
-                for layer, t in ids.items():
+                for layer, t in s.ids.items():
                     if layer not in slot['ids']:
                         slot['ids'][layer] = torch.empty(t.shape, dtype=torch.uint8).pin_memory()
                     slot['ids'][layer].copy_(t, non_blocking=True)
                 slot['done'] = torch.cuda.Event()
                 slot['done'].record(copy_stream)
-            # the device tensors must outlive the asynchronous copies
-            slot['keep'], slot['index'] = (image, stacked, ids, lat), idx
-            slot['names'] = {layer: names for layer, (names, _) in stacked.items()}
+            # the device tensors must outlive the asynchronous copies; the activations are not copied, so not held here
+            slot['keep'], slot['index'] = (s.image, s.stacked, s.ids, s.latents), s.batch_index
+            slot['names'] = {layer: names for layer, (names, _) in s.stacked.items()}
             in_flight.append(slot)
-            self.stats['pairs'] += B
-            self.stats['batches'] += 1
             n += 1
             if len(in_flight) >= depth:
                 yield finish(in_flight.pop(0))
@@ -364,13 +353,11 @@ class LabelledPairGenerator:
 
     def _iter_segmented_device(self, depth, pool, lag, cfg) -> Iterator[SegmentedBatch]:
         import collections
-        import contextlib
 
         import numpy
 
         from . import contours_device
         device = self.generator.input.input.device
-        seg = self.segmenter
         lanes = self._lanes(device)
         stages = [contours_device.DeviceContourStage(cfg) for _ in lanes]      # one workspace per lane
         B, S = self.config['batch_size'], self.generator.size
@@ -456,33 +443,14 @@ class LabelledPairGenerator:
         latent_stream = sharded_latent_stream(self.generator, self.config, self.seed, self.rank, self.world_size, self.replay_stream)
         while True:
             slot = slots[n % n_slots]
-            g, st = lanes[n % len(lanes)]
             t_enq = time.perf_counter()
-            with (torch.cuda.stream(st) if st is not None else contextlib.nullcontext()):
-                idx, latents = next(latent_stream)
-                slot['z'].copy_(latents.latent)
-                lat = Latents(slot['z'].to(device, non_blocking=True), latents.noise)
-                if self.fused_labelling:
-                    jobs = seg.make_label_jobs(g, B)
-                    acts, image = generate_images(lat, g, device=device, mean_latent=self.mean_latent, capture_layers=self.capture_layers,
-                                                  label_jobs=jobs, mix_inject_index=self.mix_inject_index)
-                    stacked = seg.jobs_to_stacked(jobs)
-                else:
-                    acts, image = generate_images(lat, g, device=device, mean_latent=self.mean_latent, capture_layers=self.capture_layers,
-                                                  mix_inject_index=self.mix_inject_index)
-                    stacked = seg.label_layers_stacked(acts)
-                if seg.keys_to_merge:
-                    stacked = seg.merge_stacked(stacked)
-                image_u8 = make_image(image)
-                slot['generated'] = torch.cuda.Event()
-                slot['generated'].record(torch.cuda.current_stream(device))
-            slot['keep'], slot['stacked'], slot['index'], slot['lane'] = (image_u8, lat, acts), stacked, idx, n % len(lanes)
+            s = self._step(lanes, n % len(lanes), latent_stream, slot['z'], image_u8=True)
+            slot['keep'], slot['stacked'], slot['index'] = (s.image, s.latents, s.activations), s.stacked, s.batch_index
+            slot['lane'], slot['generated'] = s.lane, s.event
             t_stage = time.perf_counter()
             contour_and_copy(slot)
             self.contour_stats['enqueue_generator_s'] += t_stage - t_enq
             self.contour_stats['enqueue_stage_s'] += time.perf_counter() - t_stage
-            self.stats['pairs'] += B
-            self.stats['batches'] += 1
             n += 1
             if len(pending) > max(lag, len(lanes)):
                 resolve(pending.popleft())

@@ -366,10 +366,6 @@ class ClusterSegmenter(BaseDatasetSegmenter):
         return {str(j.activation_idx): j.ids_u8 for j in jobs}
 
     @staticmethod
-    def jobs_to_margins(jobs: List[LabelJobSpec]) -> Dict[str, torch.Tensor]:
-        return {str(j.activation_idx): j.margin for j in jobs if j.margin is not None}
-
-    @staticmethod
     def jobs_to_stacked(jobs: List[LabelJobSpec]):
         return {str(j.activation_idx): (j.names, j.masks) for j in jobs}
 
@@ -385,45 +381,31 @@ class ClusterSegmenter(BaseDatasetSegmenter):
         """predict_clusters + resize_to_image_size fused: one launch per layer writes the S x S masks directly."""
         return self._as_predicted(self.label_layers_stacked(activations, class_label_map))
 
+    @staticmethod
+    def _or_masks(masks: List[torch.Tensor]) -> torch.Tensor:
+        """A new tensor: the byte-wise OR of same-shape uint8 / bool device masks (`sis_or_u8`)."""
+        acc = masks[0].contiguous().clone()
+        lib = _lib.load()
+        for m in masks[1:]:
+            m = m.contiguous()
+            with torch.cuda.device(acc.device):
+                _lib.check(lib.sis_or_u8(_lib.ptr(acc), _lib.ptr(m), acc.numel(), _lib.current_stream_ptr(acc.device)))
+        return acc
+
     def merge_sub_images(self, predicted_clusters: PredictedClusters) -> PredictedClusters:
         """OR the class masks of several layers into a destination key (black_white…segmenter.py:31-40)."""
-        lib = _lib.load()
         for dst_key, keys in self.keys_to_merge.items():
-            subs = [predicted_clusters[k] for k in keys]
-            merged = {}
-            for class_name in self.class_to_color_map:
-                acc = subs[0][class_name].contiguous().clone()
-                for s in subs[1:]:
-                    src = s[class_name].contiguous()
-                    with torch.cuda.device(acc.device):
-                        _lib.check(lib.sis_or_u8(_lib.ptr(acc), _lib.ptr(src), acc.numel(), _lib.current_stream_ptr(acc.device)))
-                merged[class_name] = acc
-            predicted_clusters[dst_key] = merged
+            predicted_clusters[dst_key] = {class_name: self._or_masks([predicted_clusters[k][class_name] for k in keys])
+                                           for class_name in self.class_to_color_map}
         return predicted_clusters
-
 
     def merge_stacked(self, stacked):
         """`merge_sub_images` on the kernel's stacked layout: adds {dst_key: (class names, uint8 [n_class, B, S, S])} for
         every `keys_to_merge` entry (class planes in `class_to_color_map` order, OR over the source layers)."""
-        lib = _lib.load()
+        names = list(self.class_to_color_map)
         for dst_key, keys in self.keys_to_merge.items():
-            names = list(self.class_to_color_map)
-            planes = []
-            for class_name in names:
-                acc = None
-                for k in keys:
-                    src_names, src = stacked[k]
-                    plane = src[src_names.index(class_name)] if class_name in src_names else None
-                    if plane is None:
-                        raise KeyError(class_name)
-                    if acc is None:
-                        acc = plane.contiguous().clone()
-                    else:
-                        plane = plane.contiguous()
-                        with torch.cuda.device(acc.device):
-                            _lib.check(lib.sis_or_u8(_lib.ptr(acc), _lib.ptr(plane), acc.numel(), _lib.current_stream_ptr(acc.device)))
-                planes.append(acc)
-            stacked[dst_key] = (names, torch.stack(planes, dim=0))
+            per_class = [dict(zip(*stacked[k])) for k in keys]        # {class name: uint8 [B, S, S] plane} per source layer
+            stacked[dst_key] = (names, torch.stack([self._or_masks([p[class_name] for p in per_class]) for class_name in names]))
         return stacked
 
     # -- host-side contour stage (contours.py; base_cluster_based…:148-450, black_white…:42-99) ------------------

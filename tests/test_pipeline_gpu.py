@@ -14,7 +14,7 @@ NAMES = {'background': '#000000', 'printed_text': '#0000FF', 'handwritten_text':
 CLASS_MAP = {'0': 'background', '1': 'printed_text', '2': 'handwritten_text', '3': 'background'}
 
 
-def make_setup(size, layers, device, precision='bf16x3', seed_centroids=5):
+def make_setup(size, layers, device, precision='bf16x3', seed_centroids=5, keys_to_merge=None):
     spec = so.GeneratorSpec(size, 512, 8, 2)
     sd = so.perturb_zero_params(so.init_state_dict(spec, seed=0), seed=1234)
     g = Generator(size, 512, 8, precision=precision)
@@ -26,7 +26,7 @@ def make_setup(size, layers, device, precision='bf16x3', seed_centroids=5):
         c, _ = g.activation_shape(int(layer))
         cents[layer] = torch.nn.functional.normalize(torch.randn(4, c, generator=gen), dim=1)
     seg = labelling.ClusterSegmenter(None, size, NAMES, keys_for_class_determination=layers[:2], keys_for_finegrained_segmentation=layers[2:],
-                                     num_clusters=4, keys_to_merge={}, catalog={k: labelling.FactorCatalog(4, v) for k, v in cents.items()},
+                                     num_clusters=4, keys_to_merge=keys_to_merge or {}, catalog={k: labelling.FactorCatalog(4, v) for k, v in cents.items()},
                                      class_label_map={k: CLASS_MAP for k in layers})
     return spec, sd, g, seg, cents
 
@@ -127,20 +127,26 @@ def test_full_size_properties(cuda_device):
 
 
 def test_iter_host_equals_device_iteration(cuda_device):
-    """The pipelined host-buffer iterator (pinned in/out, side-stream copies) returns the same pairs in order."""
+    """The pipelined host-buffer iterator (pinned in/out, side-stream copies) returns the same pairs in order, without
+    and with a `keys_to_merge` destination key (the OR of its source layers)."""
     layers = ['4', '5', '6', '7']
-    spec, sd, g, seg, cents = make_setup(32, layers, cuda_device)
     cfg = {'batch_size': 3, 'latent_size': 512}
-    ref = [b for _, b in zip(range(5), dc.LabelledPairGenerator(g, seg, cfg, seed=1))]
-    host = dc.LabelledPairGenerator(g, seg, cfg, seed=1).iter_host(depth=2)
-    for i in range(5):
-        hb = next(host)
-        assert hb.batch_index == ref[i].batch_index == i
-        assert hb.image.is_pinned() and torch.equal(hb.image, ref[i].image.cpu())
-        for layer in layers:
-            assert hb.class_names[layer] == list(NAMES)
-            for j, cn in enumerate(hb.class_names[layer]):
-                assert torch.equal(hb.masks[layer][j].bool(), ref[i].masks[layer][cn].cpu())
+    for keys_to_merge in ({}, {'merged': ['4', '6']}):
+        spec, sd, g, seg, cents = make_setup(32, layers, cuda_device, keys_to_merge=keys_to_merge)
+        ref = [b for _, b in zip(range(5), dc.LabelledPairGenerator(g, seg, cfg, seed=1))]
+        host = dc.LabelledPairGenerator(g, seg, cfg, seed=1).iter_host(depth=2)
+        for i in range(5):
+            hb = next(host)
+            assert hb.batch_index == ref[i].batch_index == i
+            assert hb.image.is_pinned() and torch.equal(hb.image, ref[i].image.cpu())
+            assert set(hb.masks) == set(ref[i].masks) == set(layers) | set(keys_to_merge)
+            for layer in hb.masks:
+                assert hb.class_names[layer] == list(NAMES)
+                for j, cn in enumerate(hb.class_names[layer]):
+                    assert torch.equal(hb.masks[layer][j].bool(), ref[i].masks[layer][cn].cpu())
+            for dst, (a, b) in keys_to_merge.items():
+                for cn in NAMES:
+                    assert torch.equal(ref[i].masks[dst][cn], ref[i].masks[a][cn] | ref[i].masks[b][cn]), (dst, cn)
 
 
 def test_in_forward_labelling_equals_separate_calls(cuda_device):
@@ -149,19 +155,22 @@ def test_in_forward_labelling_equals_separate_calls(cuda_device):
     layers = ['8', '9', '12', '13']
     spec, sd, g, seg, cents = make_setup(256, layers, cuda_device)
     cfg = {'batch_size': 4, 'latent_size': 512}
-    a = next(iter(dc.LabelledPairGenerator(g, seg, cfg, seed=3, fused_labelling=False)))
-    counts_a = {k: v.clone() for k, v in seg.cluster_pixel_counts.items()}
+    b = next(iter(dc.LabelledPairGenerator(g, seg, cfg, seed=3)))
+    counts_b = {k: v.clone() for k, v in seg.cluster_pixel_counts.items()}
     for v in seg.cluster_pixel_counts.values():
         v.zero_()
-    b = next(iter(dc.LabelledPairGenerator(g, seg, cfg, seed=3, fused_labelling=True)))
+    # the same latents and noise through the generator without label jobs, then the separate labelling launches
+    lat = next(iter(dc.build_latent_and_noise_generator(g, cfg, seed=3)))
+    acts, image = dc.generate_images(lat, g, device=cuda_device)
+    masks = seg._as_predicted(seg.label_layers_stacked(acts))
     # the fused pass sums the ToRGB channels (and, on large maps, the distances) in a different order than the separate
     # kernels: equal to rounding, not bit for bit
-    assert float((a.image - b.image).abs().max()) <= 2e-5 * float(a.image.abs().max())
+    assert float((image - b.image).abs().max()) <= 2e-5 * float(image.abs().max())
     for layer in layers:
         for cn in NAMES:
-            assert float((a.masks[layer][cn] != b.masks[layer][cn]).float().mean()) <= 1e-4, (layer, cn)
-        diff = (counts_a[layer] - seg.cluster_pixel_counts[layer]).abs().sum()
-        assert int(diff) <= 1e-4 * int(counts_a[layer].sum()), layer
+            assert float((masks[layer][cn] != b.masks[layer][cn]).float().mean()) <= 1e-4, (layer, cn)
+        diff = (seg.cluster_pixel_counts[layer] - counts_b[layer]).abs().sum()
+        assert int(diff) <= 1e-4 * int(seg.cluster_pixel_counts[layer].sum()), layer
 
 
 def test_create_segmentation_image_equals_oracle_contour_stage(cuda_device):
