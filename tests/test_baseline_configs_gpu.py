@@ -70,6 +70,16 @@ def check_batch(wl, spec, sd, g, seg, cents, class_map, batch, lat, mean_latent)
     assert agree / total >= 0.999, agree / total
     # a fused job of an activation also captured must have labelled that very tensor
     assert set(batch.activations) == set(range(spec.n_latent))
+    # every captured activation of every sample, on the kernels the batch size selects (and the plan's epilogues that
+    # write the next layer's operand planes), with test_generator_256_against_oracle's per-layer bound
+    worst_k, worst_e, worst_frac = None, 0.0, -1.0
+    for k, want in want_acts.items():
+        e = float((batch.activations[k].cpu() - want).abs().max())
+        bound = 2e-3 * max(1.0, float(want.abs().max()))
+        assert batch.activations[k].shape == want.shape and e <= bound, (k, e, bound)
+        if e / bound > worst_frac:
+            worst_k, worst_e, worst_frac = k, e, e / bound
+    print(f'\n{S}^2 B={z.shape[0]}: largest activation error {worst_e:.2e} (layer {worst_k}, {worst_frac:.3f} of its bound)')
 
 
 @pytest.mark.parametrize('cfg_id,batch_index', [(2, 1), (3, 0), (4, 0)])
