@@ -295,6 +295,53 @@ SIS_API int sis_pixel_ensemble_label(sis_pixel_ensemble* e, int n_layers, const 
                              const uint8_t* host_colors, uint8_t* d_color_image, void* stream);
 SIS_API int sis_pixel_ensemble_check(sis_pixel_ensemble* e, void* stream);
 
+/* -----------------------------------------------------------------------------------------------------------
+ * Catalog creation: steps of spherical mini-batch k-means, many independent fits per launch (one CTA per fit).
+ * Replaces the loop of MiniBatchSphericalKMeans.fit, scf/segmentation/gan_local_edit/spherical_kmeans.py:159-312
+ * (sklearn 0.24's MiniBatchKMeans on unit rows, centres renormalised after every step).  One step: renormalise the
+ * centres; reassign iff (t+1) % (10 + int(min counts)) == 0; nearest centre of each batch row; starved centres (count <
+ * ratio * max count, at most half the batch, lowest counts first) take batch rows and the smallest other count;
+ * count-weighted update; renormalise; batch inertia (mean squared distance), its EWA with alpha = min(1, 2 bs / (n+1)) in
+ * fp64, the no-improvement counter and the stop test (steps_done == max_steps, or no_improvement >= max_no_improvement
+ * when that is >= 0).
+ *
+ * Draws are counter based: h(t, j, s) = splitmix64(splitmix64(splitmix64(seed) ^ t) ^ (j << 1 | s)).  Batch row j of
+ * step t is h(t, j, 0) mod n; when centres are reassigned, the rows of the n_re smallest h(t, j, 1) (ties to the lower
+ * j) replace the starved centres in index order.  A fit's result does not depend on the other fits of a launch, nor on
+ * how its steps are split across calls.
+ *
+ * fits          : HOST array of n_fits descriptors (device pointers inside).  k in [2, 32], channels <= 512, n >= k.
+ *                 Fits may differ in n, channels and k.  Points are unit rows; centres are updated in place.
+ * d_indices     : NULL: each fit runs up to `steps` drawn steps and a fit that is done returns at once.  Otherwise
+ *                 steps must be 1 and every fit runs one step on these n_indices (<= 1024) rows: no draw, no
+ *                 reassignment, no EWA, the state is neither read nor written (d_state may be NULL).
+ * d_batch_inertia: optional [n_fits, steps] fp32, the batch inertia of each step run (entries of steps not run are
+ *                 left as they are).
+ * Asynchronous on `stream`; never synchronises.  sis_kmeans_init_state fills one fit's state (batch_size in
+ * [1, 1024], max_steps >= 1, max_no_improvement < 0 = never stop early).
+ * ----------------------------------------------------------------------------------------------------------- */
+typedef struct {
+    uint64_t seed;
+    int64_t steps_done;          /* the fit's n_iter_ */
+    int64_t max_steps;
+    int64_t done;                /* 0 running, 1 finished: the word the host polls */
+    double ewa, ewa_min;
+    int32_t batch_size, max_no_improvement, no_improvement;
+    float reassignment_ratio;
+} sis_kmeans_state;
+
+typedef struct {
+    const float* d_points; int64_t n; int channels;   /* unit rows, [n, channels] row-major */
+    int k; float* d_centers; float* d_counts;          /* [k, channels] unit rows, [k] */
+    sis_kmeans_state* d_state;                         /* per-fit state, sis_kmeans_state_bytes() */
+} sis_kmeans_fit;
+
+SIS_API int sis_kmeans_state_bytes(void);
+SIS_API int sis_kmeans_init_state(void* d_state, uint64_t seed, int batch_size, int64_t max_steps, int max_no_improvement,
+                                  float reassignment_ratio, void* stream);
+SIS_API int sis_kmeans_steps(const sis_kmeans_fit* fits, int n_fits, int steps, const int32_t* d_indices, int n_indices,
+                             float* d_batch_inertia, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

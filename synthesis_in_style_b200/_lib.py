@@ -24,6 +24,15 @@ class LabelJob(Structure):
     ]
 
 
+class KmeansFit(Structure):
+    """`sis_kmeans_fit` (include/sis_b200.h)."""
+    _fields_ = [
+        ('d_points', c_void_p), ('n', c_int64), ('channels', c_int),
+        ('k', c_int), ('d_centers', c_void_p), ('d_counts', c_void_p),
+        ('d_state', c_void_p),
+    ]
+
+
 class ForwardArgs(Structure):
     """`sis_forward_args` (include/sis_b200.h)."""
     _fields_ = [
@@ -96,6 +105,9 @@ _SIGNATURES = {
     'sis_pixel_ensemble_label': (c_int, [c_void_p, c_int, POINTER(c_void_p), POINTER(c_int), POINTER(c_int), c_int, c_int, c_void_p, c_void_p,
                                          c_void_p, c_void_p, c_void_p]),
     'sis_pixel_ensemble_check': (c_int, [c_void_p, c_void_p]),
+    'sis_kmeans_state_bytes': (c_int, []),
+    'sis_kmeans_init_state': (c_int, [c_void_p, c_uint64, c_int, c_int64, c_int, c_float, c_void_p]),
+    'sis_kmeans_steps': (c_int, [POINTER(KmeansFit), c_int, c_int, c_void_p, c_int, c_void_p, c_void_p]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
