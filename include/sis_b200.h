@@ -342,6 +342,41 @@ SIS_API int sis_kmeans_init_state(void* d_state, uint64_t seed, int batch_size, 
 SIS_API int sis_kmeans_steps(const sis_kmeans_fit* fits, int n_fits, int steps, const int32_t* d_indices, int n_indices,
                              float* d_batch_inertia, void* stream);
 
+/* -----------------------------------------------------------------------------------------------------------
+ * Training of a DatasetGAN pixel-classifier ensemble (the networks sis_pixel_ensemble_* evaluates), on the annotated
+ * pixels of generated images.  The recipe is this project's own, after DatasetGAN's train_interpreter.py:
+ *   - batches of `batch_pixels` (2..64) annotated pixels; each network draws its own order per epoch, a bijective
+ *     counter permutation of the A*S*S pixels (4-round Feistel network with cycle walking, keyed by the network's key
+ *     and the epoch: oracle/dataset_gan_train_oracle.py restates it); the trailing partial batch is dropped;
+ *   - features: every capture bilinearly upsampled to S x S at the pixel (align_corners = False), concatenated in
+ *     capture order, as the labeller; the networks run Linear, ReLU, BatchNorm1d in training mode (batch mean, biased
+ *     variance; running statistics with momentum 0.1 and the unbiased variance), ..., mean softmax cross-entropy;
+ *   - torch.optim.Adam on the 10 trainable tensors: lr 1e-3, betas (0.9, 0.999), eps 1e-8, bias correction;
+ *   - stopping: after `epochs` epochs, or, from epoch 4 on, after 51 consecutive steps whose loss is not below the
+ *     network's best.  fp32 arithmetic with fixed summation orders: a network's result depends neither on the other
+ *     networks of the trainer nor on how its steps are split into calls.
+ * create       : 1..8 networks, 2 <= n_class < 32, feature_size a positive multiple of 32.
+ * set_param    : initial values per network under the state-dict keys of sis_pixel_ensemble_set_param (HOST memory).
+ * set_data     : captures fp32 NCHW [n_images, C_l, r_l, r_l] and labels uint8 [n_images, S, S] (ids < n_class) on
+ *                the device; they must stay alive and unchanged while the trainer runs.  n_images * S * S <= 2^31 - 1.
+ * prepare      : uploads the parameters, zeroes the optimiser state; keys[m] is network m's draw key.
+ * steps        : enqueues `steps` steps for every network that has not stopped; never synchronises.
+ * status       : synchronises `stream`; done[m] (0/1) and steps_done[m] (= num_batches_tracked) per network.
+ * read_param   : the current value of a state-dict key (running statistics included) into HOST memory.
+ * read_losses  : the first `count` (<= steps_done) per-step losses of a network into HOST memory.
+ * ----------------------------------------------------------------------------------------------------------- */
+typedef struct sis_pixel_train sis_pixel_train;
+SIS_API int sis_pixel_train_create(sis_pixel_train** out, int n_models, int feature_size, int n_class, int batch_pixels);
+SIS_API void sis_pixel_train_destroy(sis_pixel_train* t);
+SIS_API int sis_pixel_train_set_param(sis_pixel_train* t, int model, const char* name, const float* host_data, int64_t numel);
+SIS_API int sis_pixel_train_set_data(sis_pixel_train* t, int n_layers, const float* const* d_activations, const int* channels,
+                                     const int* resolutions, int n_images, int image_size, const uint8_t* d_labels);
+SIS_API int sis_pixel_train_prepare(sis_pixel_train* t, const uint64_t* keys, int epochs, void* stream);
+SIS_API int sis_pixel_train_steps(sis_pixel_train* t, int steps, void* stream);
+SIS_API int sis_pixel_train_status(sis_pixel_train* t, int32_t* done, int64_t* steps_done, void* stream);
+SIS_API int sis_pixel_train_read_param(sis_pixel_train* t, int model, const char* name, float* host_out, int64_t numel, void* stream);
+SIS_API int sis_pixel_train_read_losses(sis_pixel_train* t, int model, float* host_out, int64_t count, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -105,6 +105,15 @@ _SIGNATURES = {
     'sis_pixel_ensemble_label': (c_int, [c_void_p, c_int, POINTER(c_void_p), POINTER(c_int), POINTER(c_int), c_int, c_int, c_void_p, c_void_p,
                                          c_void_p, c_void_p, c_void_p]),
     'sis_pixel_ensemble_check': (c_int, [c_void_p, c_void_p]),
+    'sis_pixel_train_create': (c_int, [POINTER(c_void_p), c_int, c_int, c_int, c_int]),
+    'sis_pixel_train_destroy': (None, [c_void_p]),
+    'sis_pixel_train_set_param': (c_int, [c_void_p, c_int, c_char_p, c_void_p, c_int64]),
+    'sis_pixel_train_set_data': (c_int, [c_void_p, c_int, POINTER(c_void_p), POINTER(c_int), POINTER(c_int), c_int, c_int, c_void_p]),
+    'sis_pixel_train_prepare': (c_int, [c_void_p, POINTER(c_uint64), c_int, c_void_p]),
+    'sis_pixel_train_steps': (c_int, [c_void_p, c_int, c_void_p]),
+    'sis_pixel_train_status': (c_int, [c_void_p, POINTER(ctypes.c_int32), POINTER(c_int64), c_void_p]),
+    'sis_pixel_train_read_param': (c_int, [c_void_p, c_int, c_char_p, c_void_p, c_int64, c_void_p]),
+    'sis_pixel_train_read_losses': (c_int, [c_void_p, c_int, c_void_p, c_int64, c_void_p]),
     'sis_kmeans_state_bytes': (c_int, []),
     'sis_kmeans_init_state': (c_int, [c_void_p, c_uint64, c_int, c_int64, c_int, c_float, c_void_p]),
     'sis_kmeans_steps': (c_int, [POINTER(KmeansFit), c_int, c_int, c_void_p, c_int, c_void_p, c_void_p]),

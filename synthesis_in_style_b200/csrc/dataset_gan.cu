@@ -18,13 +18,12 @@
 #include <vector>
 #include <cmath>
 #include "common.cuh"
+#include "dataset_gan_common.cuh"
 #include "kernels.h"
 #include "modconv_tc.h"
 #include "../../include/sis_b200.h"
 
 namespace sis {
-
-constexpr int GAN_H1 = 128, GAN_H2 = 32, GAN_MAX_GROUPS = 8, GAN_MAX_MODELS = 8;
 
 struct GanTailArgs {
     const float* y[GAN_MAX_GROUPS];     // first-layer products per resolution: fp32 [B][M*128][r][r] (NCHW) or, when
@@ -78,14 +77,9 @@ __global__ void __launch_bounds__(128) dataset_gan_tail_kernel(GanTailArgs a) {
 #pragma unroll
                 for (int i = 0; i < GAN_H1; ++i) z[i] += __ldg(q + (int64_t)i * plane);
             } else {
-                // nn.Upsample(scale_factor = S / r, mode='bilinear'), align_corners = False:
-                // src = max((dst + 0.5) * r / S - 0.5, 0), i0 = floor(src), i1 = min(i0 + 1, r - 1)
-                const float sc = (float)r / (float)a.S;
-                const float fy = fmaxf(((float)oy + 0.5f) * sc - 0.5f, 0.0f), fx = fmaxf(((float)ox + 0.5f) * sc - 0.5f, 0.0f);
-                const int y0 = (int)fy, x0 = (int)fx;
-                const int y1 = min(y0 + 1, r - 1), x1 = min(x0 + 1, r - 1);
-                const float ly = fy - (float)y0, lx = fx - (float)x0;
-                const float w00 = (1.0f - ly) * (1.0f - lx), w01 = (1.0f - ly) * lx, w10 = ly * (1.0f - lx), w11 = ly * lx;
+                const GanBilinearTap tap = gan_bilinear_tap(oy, ox, r, a.S);
+                const int y0 = tap.y0, y1 = tap.y1, x0 = tap.x0, x1 = tap.x1;
+                const float w00 = tap.w00, w01 = tap.w01, w10 = tap.w10, w11 = tap.w11;
                 const float* q00 = base + y0 * r + x0; const float* q01 = base + y0 * r + x1;
                 const float* q10 = base + y1 * r + x0; const float* q11 = base + y1 * r + x1;
 #pragma unroll
@@ -234,13 +228,9 @@ __global__ void __launch_bounds__(128, 4) dataset_gan_tail_tiled_kernel(GanTailA
                 gan_src_range(ox0, GAN_TX, r, a.S, fx0, fx1);
                 const int fw = fx1 - fx0 + 1;
                 const float* src = s_src + base_px[g] * GAN_SRC_STRIDE;
-                // nn.Upsample(scale_factor = S / r, mode='bilinear'), align_corners = False
-                const float sc = (float)r / (float)a.S;
-                const float fy = fmaxf(((float)oy + 0.5f) * sc - 0.5f, 0.0f), fx = fmaxf(((float)ox + 0.5f) * sc - 0.5f, 0.0f);
-                const int y0 = (int)fy, x0 = (int)fx;
-                const int y1 = min(y0 + 1, r - 1), x1 = min(x0 + 1, r - 1);
-                const float ly = fy - (float)y0, lx = fx - (float)x0;
-                const float w00 = (1.0f - ly) * (1.0f - lx), w01 = (1.0f - ly) * lx, w10 = ly * (1.0f - lx), w11 = ly * lx;
+                const GanBilinearTap tap = gan_bilinear_tap(oy, ox, r, a.S);
+                const int y0 = tap.y0, y1 = tap.y1, x0 = tap.x0, x1 = tap.x1;
+                const float w00 = tap.w00, w01 = tap.w01, w10 = tap.w10, w11 = tap.w11;
                 const float4* q00 = reinterpret_cast<const float4*>(src + ((y0 - fy0) * fw + x0 - fx0) * GAN_SRC_STRIDE);
                 const float4* q01 = reinterpret_cast<const float4*>(src + ((y0 - fy0) * fw + x1 - fx0) * GAN_SRC_STRIDE);
                 const float4* q10 = reinterpret_cast<const float4*>(src + ((y1 - fy0) * fw + x0 - fx0) * GAN_SRC_STRIDE);
